@@ -4,6 +4,7 @@ bench.py -- headline measurement: fp64 ray*surfaces/s of the fused trace on N B2
 
     python bench.py [--gpus N] [--steps K] [--warmup W]              # this framework (one rank per GPU under torchrun)
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]   # the reference algorithm on the host cores
+    python bench.py ... --dump-outputs DIR      # also save what the last timed step computed (see dump_outputs)
 
 Workload (BASELINE.json config 5 / north star): the 10-surface achromat relay of
 scripts/2022_08_24_relay_astigmatism.py (8 spherical + 2 flat surfaces, 6 Sellmeier + 3 constant media, 0.785 um),
@@ -321,6 +322,29 @@ def cpu_baseline_run(n_threads: int, target_seconds: float = 12.0):
     return best, f"{side}x{side} = {side * side} rays x {N_SURFACES} surfaces, final slab only, best of 2"
 
 
+def dump_outputs(path: Path, out, reducer, n_rows: int = 1 << 18, n_cells: int = 1 << 20):
+    """What the timed step hands its caller, as finite float64 .npy files (42 MB at most) for comparing two builds
+    output for output.  A fixed seeded sample of the final slab's rays (in index order) is split in two, since the
+    trace marks a ray that leaves the system (outside an aperture, total internal reflection) with NaN:
+    final_slab_alive.npy, 1 or 0 per sampled ray for whether its whole row is finite, and final_slab.npy, the rows of
+    the sampled rays that came through.  spot_stats.npy holds the spot statistics; pupil_grid.npy, a fixed seeded
+    sample of the pupil grid's cells, (3 planes, cells)."""
+    import torch
+    path.mkdir(parents=True, exist_ok=True)
+    n = out.shape[1]
+    rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, n_rows), replace=False))
+    slab = out[0, torch.as_tensor(rows, device=out.device)].cpu().numpy()
+    alive = np.isfinite(slab).all(axis=1)
+    np.save(path / "final_slab_alive.npy", alive.astype(np.float64))
+    np.save(path / "final_slab.npy", slab[alive])
+    if reducer is not None and reducer.stats_t is not None:
+        np.save(path / "spot_stats.npy", reducer.stats_t.cpu().numpy())
+    if reducer is not None and reducer.grid_t is not None:
+        grid = reducer.grid_t.reshape(3, -1)
+        cells = np.sort(np.random.default_rng(1).choice(grid.shape[1], size=min(grid.shape[1], n_cells), replace=False))
+        np.save(path / "pupil_grid.npy", grid[:, torch.as_tensor(cells, device=out.device)].cpu().numpy())
+
+
 WORKLOAD = ("relay10 (BASELINE config 5 system): 10-surface achromat relay, 0.785 um, collimated Cartesian bundle, "
             "final slab + fused pupil reduction")
 
@@ -390,7 +414,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config block (BASELINE configs 1-5, N = 1)")
     ap.add_argument("--no-bind", action="store_true", help="do not pin each rank to its GPU's local CPUs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -545,6 +572,8 @@ def main():
     n_valid = int(torch.isfinite(out[0, :, 0]).sum())
     last = reducers[(args.steps - 1) % len(reducers)] if reducers else None
     stats = last.stats() if (last is not None and last.stats_t is not None) else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(Path(args.dump_outputs), out, last)
 
     # ---- the reference's own output mode (full (2S+1, N, 8) history), device resident: the HBM-bound regime ------
     full_history = None
@@ -611,7 +640,7 @@ def main():
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
     t0 = time.perf_counter()
     for _ in range(e2e_steps):
         engine.trace_host(system.surfaces, materials, host_in, keep="last", device=local, out=host_out)

@@ -30,12 +30,12 @@ def test_library_loads_and_exports_every_declared_symbol():
     assert L.rtb_abi_version() == _ffi.RTB_ABI_VERSION
 
 
-def test_struct_layouts_match_the_header():
+def test_struct_layouts_match_the_header(tmp_path):
     """sizes the C compiler gives the header's structs == ctypes' sizes"""
     from ray_trace_pb_b200 import _ffi
     src = ('#include <stdio.h>\n#include "rtb.h"\nint main(){printf("%zu %zu %zu %zu %zu %zu\\n", sizeof(rtb_surface),'
            'sizeof(rtb_material), sizeof(rtb_system), sizeof(rtb_reduce), sizeof(rtb_trace_opts), sizeof(rtb_source));}')
-    exe = Path("/tmp/rtb_sizes")
+    exe = tmp_path / "rtb_sizes"
     subprocess.run(["gcc", "-x", "c", "-", "-I", str(ROOT / "include"), "-o", str(exe)], input=src.encode(), check=True)
     sizes = [int(v) for v in subprocess.run([str(exe)], capture_output=True, check=True).stdout.split()]
     want = [ctypes.sizeof(c) for c in (_ffi.RtbSurface, _ffi.RtbMaterial, _ffi.RtbSystem, _ffi.RtbReduce,

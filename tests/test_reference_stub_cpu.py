@@ -1,58 +1,59 @@
 """
 CPU test (no GPU): the ctypes stub of INTEGRATION.md section 2 (tests/reference_stub.py) run against the REAL reference
-classes -- the unmodified package in baseline/_ref/ (installed by baseline/install_ref.sh in the build container and
-shipped with the snapshot; /root/reference/src is the fallback there) -- up to, and not including, the device call:
-every struct the stub packs from the reference's own objects must equal, byte for byte, what this framework's host
-layer packs from its mirror of the same system, and the refractive-index tables must be the same bits.
-Skipped where the reference is not installed.
+objects -- as recorded in the golden cases by tests/golden/make_golden.py: every attribute the stub reads from the
+reference's surfaces (the case's `system` prescription) and the reference media's n() at the case's wavelengths
+(`n_table`) -- up to, and not including, the device call: every struct the stub packs from them must equal, byte for
+byte, what this framework's host layer packs from its mirror of the same system, and the refractive-index tables must
+be the same bits.
 """
 import ctypes
-import sys
-import types
-from pathlib import Path
+import json
+from types import SimpleNamespace
 
 import numpy as np
 import pytest
 
 import systems
+from conftest import load_golden
 
-ROOT = Path(__file__).resolve().parent.parent
+
+class RecordedMedium:
+    """One of the reference's media, answering n() with the values recorded from it.  The stub also asks for n(NaN);
+    where a case did not record that column, the reference's rule applies, as edge_mix's table records it: a Constant
+    gives its index, every Sellmeier medium (Vacuum included) NaN."""
+
+    def __init__(self, desc, wavelengths, values):
+        self.known = dict(zip(wavelengths.tolist(), values.tolist()))
+        recorded = [v for w, v in self.known.items() if np.isnan(w)]
+        self.at_nan = recorded[0] if recorded else (desc["n"] if desc["type"] == "Constant" else np.nan)
+
+    def n(self, wavelength):
+        return np.array([self.at_nan if np.isnan(w) else self.known[w] for w in np.asarray(wavelength).reshape(-1)])
 
 
-def _reference_modules():
-    for base in (ROOT / "baseline" / "_ref", Path("/root/reference/src")):
-        if (base / "raytrace" / "raytrace.py").exists():
-            break
-    else:
-        pytest.skip("the reference is not installed (baseline/install_ref.sh)")
-    for name in ("matplotlib", "matplotlib.figure", "matplotlib.axes", "matplotlib.axes._axes", "matplotlib.pyplot"):
-        sys.modules.setdefault(name, types.ModuleType(name))
-    sys.modules["matplotlib.figure"].Figure = object
-    sys.modules["matplotlib.axes._axes"].Axes = object
-    saved = {k: sys.modules.pop(k) for k in [k for k in sys.modules if k == "raytrace" or k.startswith("raytrace.")]}
-    sys.path.insert(0, str(base))
-    try:
-        import raytrace.materials as ref_rtm
-        import raytrace.raytrace as ref_rt
-        assert Path(ref_rt.__file__).resolve().is_relative_to(base.resolve())
-    finally:
-        sys.path.remove(str(base))
-        for k in [k for k in sys.modules if k == "raytrace" or k.startswith("raytrace.")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
-    return ref_rt, ref_rtm
+def recorded_reference(name):
+    """(system, m_in, m_out, rays) of a golden case, standing in for the reference's own objects"""
+    g = load_golden(name)
+    desc = json.loads(str(g["system"]))
+    surfaces = []
+    for d in desc["surfaces"]:
+        s = type(d["type"], (), {})()                  # the stub dispatches on the class name
+        s.__dict__.update({k: np.array(v) if isinstance(v, list) else v for k, v in d.items() if k != "type"})
+        surfaces.append(s)
+    media = [desc["initial_material"]] + desc["materials"] + [desc["final_material"]]
+    media = [RecordedMedium(m, g["unique_wavelengths"], g["n_table"][:, k]) for k, m in enumerate(media)]
+    return SimpleNamespace(surfaces=surfaces, materials=media[1:-1]), media[0], media[-1], g["rays_in"], desc
 
 
 @pytest.mark.parametrize("builder", ["relay10", "opm", "edge_mix", "doublet_nlak22", "mirrors", "reversed_doublet"])
 def test_stub_packs_the_real_reference_classes(builder, rt, rtm):
     import reference_stub
     from ray_trace_pb_b200 import engine
-    ref_rt, ref_rtm = _reference_modules()
-    system, m_in, m_out, rays = getattr(systems, builder)(ref_rt, ref_rtm)            # the reference's own objects
+    system, m_in, m_out, rays, desc = recorded_reference(builder)                    # the reference's own values
     sysd, packed_rays, _keep = reference_stub.pack(system, rays, m_in, m_out)
     assert sysd.n_surfaces == len(system.surfaces) and packed_rays.shape == (len(rays), 8)
 
-    mirror, mm_in, mm_out = systems.rebuild_system(systems.describe_system(system, m_in, m_out), rt, rtm)
+    mirror, mm_in, mm_out = systems.rebuild_system(desc, rt, rtm)
     wl = np.unique(rays[~np.isnan(rays[:, 7]), 7])
     ours = engine.pack_system(mirror.surfaces, [mm_in] + mirror.materials + [mm_out], wl)
     assert ours.sys.n_surfaces == sysd.n_surfaces and ours.sys.n_wavelengths == sysd.n_wavelengths
