@@ -228,6 +228,9 @@ __global__ void __launch_bounds__(256) exact_math_selftest_kernel(unsigned long 
 {
     const long long stride = (long long)gridDim.x * blockDim.x;
     unsigned long long bad_div = 0, bad_div3 = 0, bad_sqrt = 0;
+    __shared__ double2 near_one_tab[xm::kNearOneEntries];
+    for (int k = threadIdx.x; k < xm::kNearOneEntries; k += blockDim.x) near_one_tab[k] = xm::near_one_entry(k);
+    __syncthreads();
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         const int cat = (int)(i & 3);
         const unsigned long long h0 = splitmix64(seed ^ (unsigned long long)(4 * i));
@@ -244,6 +247,18 @@ __global__ void __launch_bounds__(256) exact_math_selftest_kernel(unsigned long 
         bad_div3 += !(same_bits(x, a0 / b) && same_bits(y, a1 / b) && same_bits(z, a2 / b));
         bad_sqrt += !same_bits(xm::sqrt(a0), sqrt(a0));
         bad_sqrt += !same_bits(xm::sqrt(fabs(a2)), sqrt(fabs(a2)));
+        // the near-one table: every s = bits(1.0) + k, k in [-128, 127], passes, and a numerator of moderate size (those
+        // of lean_steps.cuh are components of a vector of norm sqrt(s)) is divided by it as c / sqrt(s) divides; the
+        // doubles next to either end of the table fail
+        const long long k = (long long)((i >> 2) & (xm::kNearOneEntries - 1)) - xm::kNearOneEntries / 2;
+        const double s = __longlong_as_double(0x3FF0000000000000ll + k);
+        const double c = (cat & 1) ? a0 : test_operand(splitmix64(h0 + 4), 1);
+        bool in = true, below = true, above = true;
+        const double2 lr = xm::near_one(in, s, near_one_tab);
+        xm::near_one(below, __longlong_as_double(0x3FF0000000000000ll - xm::kNearOneEntries / 2 - 1), near_one_tab);
+        xm::near_one(above, __longlong_as_double(0x3FF0000000000000ll + xm::kNearOneEntries / 2), near_one_tab);
+        bad_div += !in | below | above;
+        if (xm::num_ok(c)) bad_div += !same_bits(xm::div_core(c, lr.x, lr.y), c / sqrt(s));
     }
     if (bad_div) atomicAdd(bad + 0, bad_div);
     if (bad_div3) atomicAdd(bad + 1, bad_div3);

@@ -72,6 +72,7 @@ struct __align__(16) SurfaceShared {
 
 struct LeanShared {
     SurfaceShared surf[kMaxSurfaces];
+    double2 near_one[xm::kNearOneEntries];  // (sqrt(s), 1/sqrt(s)) for |c|^2 = s near 1 (exact_math.cuh)
     int run_clean[kMaxSurfaces + 2];      // the probe overrode no surface of this run (see TraceParams::lean_run_*)
 };
 
@@ -264,6 +265,7 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
         for (int k = 0; k < 12; k++)
             s_tally[tally_index(k, threadIdx.x)] = (k < 8) ? 0.0 : ((k == 8 || k == 10) ? CUDART_INF : -CUDART_INF);
     }
+    for (int k = threadIdx.x; k < xm::kNearOneEntries; k += blockDim.x) s_c.near_one[k] = xm::near_one_entry(k);
     for (int k = threadIdx.x; k < P.n_surf; k += blockDim.x) {
         const DevSurface &s = P.surf[k];
         const double den = (s.kind == RTB_SURF_PERFECT_LENS) ? s.focal_len : s.radius;
@@ -373,7 +375,7 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
                         const double n2 = USE_TABLE ? 0.0 : eval_index(P.mat[k + 1], wl0);
                         const double ratio = USE_TABLE ? pair[-1] : xm::div(n1, n2);
                         bool ok = true, kill;
-                        const bool on = lean::sphere_axial(ok, P.surf[k], s_c.surf[k].rcp, r, n1, ratio, wl0, wl_rcp, kill);
+                        const bool on = lean::sphere_axial(ok, P.surf[k], s_c.surf[k].rcp, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                         failed = failed | (alive & !ok);
                         at_valid = alive & ok & !kill;
                         alive = alive & ok & on;
@@ -392,7 +394,7 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
                         const double n2 = USE_TABLE ? 0.0 : eval_index(P.mat[k + 1], wl0);
                         const double ratio = USE_TABLE ? pair[-1] : xm::div(n1, n2);
                         bool ok = true, kill;
-                        const bool on = lean::flat_axial<false>(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, kill);
+                        const bool on = lean::flat_axial<false>(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                         failed = failed | (alive & !ok);
                         at_valid = alive & ok & !kill;
                         alive = alive & ok & on;
@@ -413,7 +415,7 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
                         const double n2 = USE_TABLE ? 0.0 : eval_index(P.mat[k + 1], wl0);
                         const double ratio = USE_TABLE ? pair[-1] : xm::div(n1, n2);
                         bool ok = true, kill;
-                        const bool on = lean::flat_axial<true>(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, kill);
+                        const bool on = lean::flat_axial<true>(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                         failed = failed | (alive & !ok);
                         at_valid = alive & ok & !kill;
                         alive = alive & ok & on;
@@ -432,7 +434,7 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
                         const double n2 = USE_TABLE ? 0.0 : eval_index(P.mat[k + 1], wl0);
                         const double ratio = USE_TABLE ? pair[-1] : xm::div(n1, n2);
                         bool ok = true, kill;
-                        const bool on = lean::flat_any(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, kill);
+                        const bool on = lean::flat_any(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                         failed = failed | (alive & !ok);
                         at_valid = alive & ok & !kill;
                         alive = alive & ok & on;
@@ -532,13 +534,13 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
                         bool ok = true, kill;
                         bool on;
                         if (ss.code == kLeanSphere) {
-                            on = lean::sphere_axial(ok, s, ss.rcp, r, n1, ratio, wl0, wl_rcp, kill);
+                            on = lean::sphere_axial(ok, s, ss.rcp, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                         } else if (ss.code == kLeanFlat) {
-                            on = lean::flat_axial<false>(ok, s, r, n1, ratio, wl0, wl_rcp, kill);
+                            on = lean::flat_axial<false>(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                         } else if (ss.code == kLeanFlatZ) {
-                            on = lean::flat_axial<true>(ok, s, r, n1, ratio, wl0, wl_rcp, kill);
+                            on = lean::flat_axial<true>(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                         } else if (KINDS == 1 && ss.code == kLeanFlatAny) {
-                            on = lean::flat_any(ok, s, r, n1, ratio, wl0, wl_rcp, kill);
+                            on = lean::flat_any(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                         } else if (KINDS == 1 && ss.code == kLeanLens) {
                             on = lean::lens_any(ok, s, ss.rcp, r, n1, n2, wl0, wl_rcp);
                             kill = false;
@@ -580,13 +582,13 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
                 const lean::State before = r;
                 bool ok = true, on, kill;
                 if (code == kLeanSphere)
-                    on = lean::sphere_axial(ok, s, ss.rcp, r, n1, ratio, wl0, wl_rcp, kill);
+                    on = lean::sphere_axial(ok, s, ss.rcp, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                 else if (code == kLeanFlat)
-                    on = lean::flat_axial<false>(ok, s, r, n1, ratio, wl0, wl_rcp, kill);
+                    on = lean::flat_axial<false>(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                 else if (code == kLeanFlatZ)
-                    on = lean::flat_axial<true>(ok, s, r, n1, ratio, wl0, wl_rcp, kill);
+                    on = lean::flat_axial<true>(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                 else if (code == kLeanFlatAny)
-                    on = lean::flat_any(ok, s, r, n1, ratio, wl0, wl_rcp, kill);
+                    on = lean::flat_any(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
                 else if (code == kLeanLens)
                     on = lean::lens_any(ok, s, ss.rcp, r, n1, n2, wl0, wl_rcp);
                 else
