@@ -25,6 +25,26 @@ __device__ __forceinline__ double eval_index(const DevMaterial &m, double wl)
 // a ray whose wavelength is not in the host table (the table may be built from a sample of the batch)
 static __device__ __noinline__ double index_for_unlisted(const DevMaterial *m, double wl) { return eval_index(*m, wl); }
 
+// the row of the index tables that lists wavelength wl (bit for bit), or P.n_wl -- the NaN-wavelength row -- when none does
+__device__ __forceinline__ int wavelength_row(const TraceParams &P, double wl)
+{
+    int row = P.n_wl;
+    const long long bits = __double_as_longlong(wl);
+#pragma unroll 1
+    for (int k = 0; k < P.n_wl; k++)
+        if (__double_as_longlong(P.wl[k]) == bits) row = k;
+    return row;
+}
+
+// a reciprocal 1/den usable by the optimistic steps: finite, |den| < 2^52, and a reciprocal that is an ordinary normal
+// number
+__device__ __forceinline__ bool usable_rcp(double den, double rcp)
+{
+    return xm::den_ok(den) && fabs(den) < 4503599627370496.0 && xm::quo_ok(rcp);
+}
+
+__device__ __forceinline__ bool non_finite(double v) { return (__double2hiint(v) & 0x7ff00000) == 0x7ff00000; }
+
 // ---- ray I/O ---------------------------------------------------------------------------------------------
 // Two layouts (rtb_trace_opts.flags): rows of 8 doubles -- the reference's (N, 8), moved as two 256-bit accesses per
 // ray so every 32-byte sector is used whole -- or planes (8, N), where each of the eight accesses of a warp is one

@@ -42,10 +42,6 @@ struct SharedConsts {
     unsigned long long rcp_ok;       // bit k: that reciprocal is usable by the Optimistic steps (see below)
 };
 
-// The final-slab-only kernel's surface step as a FUNCTION: it must be inlined at both of its call sites -- out of line,
-// the prescription would be read through generic pointers into the parameter block, at half the speed -- and only
-// functions can be forced (the general kernel's lambda below is inlined by the compiler's own choice, and that
-// kernel's register allocation does not take kindly to being rearranged).
 struct RayLoop {       // the loop-carried state of one ray
     Ray cur;
     double n1, n2;     // refractive index before / after the current surface
@@ -57,17 +53,37 @@ struct RayLoop {       // the loop-carried state of one ray
     bool force_careful;
 };
 
-template <class OPT, bool USE_TABLE>
+// the refractive index after surface kk
+template <bool USE_TABLE>
+__device__ __forceinline__ double index_after(const TraceParams &P, const double *s_ntab, int kk, const RayLoop &st)
+{
+    return !USE_TABLE ? eval_index(P.mat[kk + 1], st.wl0)
+                      : (st.unlisted ? index_for_unlisted(&P.mat[kk + 1], st.wl0) : s_ntab[st.row + kk + 1]);
+}
+
+// 1/R (1/f for a perfect lens) of surface kk
+__device__ __forceinline__ xm::Rcp radius_rcp(const DevSurface &s, const SharedConsts &s_c, int kk)
+{
+    xm::Rcp r;
+    r.b = (s.kind == RTB_SURF_PERFECT_LENS) ? s.focal_len : s.radius;
+    r.y = s_c.rcp_radius[kk];
+    r.ok = (s_c.rcp_ok >> kk) & 1ull;
+    return r;
+}
+
+// One surface with nothing to keep.  It runs optimistically; one flag says whether every intermediate stayed in the fast
+// paths' domain, otherwise the surface is redone with the Careful arithmetic (surface_steps.cuh).  (Each kind's redo
+// sits in its own branch: one careful_step after the branches costs the final-slab kernels 34 FP64 instructions and
+// spill traffic.)
+// A FUNCTION: it must be inlined at every call site -- out of line, the prescription would be read through generic
+// pointers into the parameter block, at half the speed -- and only functions can be forced.
+template <class OPT, bool USE_TABLE, bool INTERSECT_ONLY>
 __device__ __forceinline__ void plain_surface_step(const TraceParams &P, const double *s_ntab, const double *s_ratio,
                                                    const SharedConsts &s_c, int kk, RayLoop &st)
 {
     const DevSurface &s = P.surf[kk];
-    st.n2 = !USE_TABLE ? eval_index(P.mat[kk + 1], st.wl0)
-                       : (st.unlisted ? index_for_unlisted(&P.mat[kk + 1], st.wl0) : s_ntab[st.row + kk + 1]);
-    xm::Rcp rcp_k;
-    rcp_k.b = (s.kind == RTB_SURF_PERFECT_LENS) ? s.focal_len : s.radius;
-    rcp_k.y = s_c.rcp_radius[kk];
-    rcp_k.ok = (s_c.rcp_ok >> kk) & 1ull;
+    st.n2 = index_after<USE_TABLE>(P, s_ntab, kk, st);
+    const xm::Rcp rcp_k = radius_rcp(s, s_c, kk);
     OPT m;
     m.ok = !st.force_careful;
     st.force_careful = false;
@@ -75,9 +91,9 @@ __device__ __forceinline__ void plain_surface_step(const TraceParams &P, const d
     Ray after;
     if (s.kind == RTB_SURF_FLAT || s.kind == RTB_SURF_SPHERE) {
         const double ratio = (USE_TABLE && !st.unlisted) ? s_ratio[st.row + kk] : xm::div(st.n1, st.n2);
-        st.dead = refracting_step<OPT, false>(m, s, st.cur, st.n1, ratio, st.rcp_wl, rcp_k, true, raw, after);
+        st.dead = refracting_step<OPT, false>(m, s, st.cur, st.n1, ratio, st.rcp_wl, rcp_k, !INTERSECT_ONLY, raw, after);
         if (!m.ok) {
-            const StepResult redo = careful_refracting(&s, st.cur, st.n1, ratio, true);
+            const StepResult redo = careful_refracting(&s, st.cur, st.n1, ratio, !INTERSECT_ONLY);
             after = redo.after;
             st.dead = redo.dead;
         }
@@ -89,9 +105,9 @@ __device__ __forceinline__ void plain_surface_step(const TraceParams &P, const d
             st.dead = redo.dead;
         }
     } else {
-        st.dead = perfect_lens_step<OPT>(m, s, st.cur, st.n1, st.n2, st.rcp_wl, rcp_k, false, false, raw, after);
+        st.dead = perfect_lens_step<OPT>(m, s, st.cur, st.n1, st.n2, st.rcp_wl, rcp_k, INTERSECT_ONLY, false, raw, after);
         if (!m.ok) {
-            const StepResult redo = careful_lens(&s, st.cur, st.n1, st.n2, false);
+            const StepResult redo = careful_lens(&s, st.cur, st.n1, st.n2, INTERSECT_ONLY);
             after = redo.after;
             st.dead = redo.dead;
         }
@@ -141,9 +157,7 @@ __global__ void __launch_bounds__(kTraceThreads, kTraceMinBlocks) trace_f64_kern
         const DevSurface &s = P.surf[k];
         const double den = (s.kind == RTB_SURF_PERFECT_LENS) ? s.focal_len : s.radius;
         s_c.rcp_radius[k] = xm::refine_rcp(den);
-        // usable by the Optimistic steps: finite, |den| < 2^52, and a reciprocal that is an ordinary normal number
-        const bool sane = xm::den_ok(den) && fabs(den) < 4503599627370496.0 && xm::quo_ok(s_c.rcp_radius[k]);
-        if (sane) atomicOr(&s_c.rcp_ok, 1ull << k);
+        if (usable_rcp(den, s_c.rcp_radius[k])) atomicOr(&s_c.rcp_ok, 1ull << k);
     }
     __syncthreads();
 
@@ -168,193 +182,118 @@ __global__ void __launch_bounds__(kTraceThreads, kTraceMinBlocks) trace_f64_kern
             load_ray(P.rays_in, i, P.n_rays, planes_in, cur);
 
         // refractive indices are functions of the launch wavelength; see DESIGN.md ("n is taken at launch")
-        const double wl0 = cur.wl;
-        const xm::Rcp rcp_wl = xm::make_rcp(wl0);
-        int row = 0;
-        bool unlisted = false;
+        RayLoop st;
+        st.cur = cur;
+        st.wl0 = cur.wl;
+        st.rcp_wl = xm::make_rcp(st.wl0);
+        st.row = 0;
+        st.unlisted = false;
         if (USE_TABLE) {
-            row = P.n_wl; // the NaN-wavelength row
-            const long long bits = __double_as_longlong(wl0);
-#pragma unroll 1
-            for (int k = 0; k < P.n_wl; k++)
-                if (__double_as_longlong(P.wl[k]) == bits) row = k;
+            const int row = wavelength_row(P, st.wl0);
             // a valid wavelength the table does not list: evaluate Sellmeier / constant media for this ray
-            unlisted = (row == P.n_wl) && (wl0 == wl0);
-            row *= n_med;
+            st.unlisted = (row == P.n_wl) && (st.wl0 == st.wl0);
+            st.row = row * n_med;
         }
         if (GENERAL) {
             if (P.slab_pos[0] >= 0) store_ray(P.out + P.slab_pos[0] * P.out_stride, row0 + i, out_rows, planes_out, cur);
             if (reducing && P.red.slab == 0) reduce_sample(red, cur, tally);
         }
 
-        double n1 = !USE_TABLE ? eval_index(P.mat[0], wl0)
-                               : (unlisted ? index_for_unlisted(&P.mat[0], wl0) : s_ntab[row]);
+        st.n1 = !USE_TABLE ? eval_index(P.mat[0], st.wl0)
+                           : (st.unlisted ? index_for_unlisted(&P.mat[0], st.wl0) : s_ntab[st.row]);
+        st.n2 = st.n1;
         // Live rays run the surface loop; a ray that dies (leaves a surface all-NaN) drops out of it and only has
         // its remaining slabs blanked below -- an all-NaN ray stays all-NaN through every kind of surface.
-        bool dead = false;
+        st.dead = false;
         // The optimistic steps may assume finite geometry (that is what licenses their shortcuts), and inside a trace
         // it always is -- the reference blanks x, y, z together.  Only a ray that ARRIVES with an inf/NaN in some
         // position or direction column could break that, so such a ray takes the careful path at its first surface.
-        auto non_finite = [](double v) { return (__double2hiint(v) & 0x7ff00000) == 0x7ff00000; };
-        bool force_careful = non_finite(cur.ox) | non_finite(cur.oy) | non_finite(cur.oz) | non_finite(cur.dx) |
-                             non_finite(cur.dy) | non_finite(cur.dz);
+        st.force_careful = non_finite(cur.ox) | non_finite(cur.oy) | non_finite(cur.oz) | non_finite(cur.dx) |
+                           non_finite(cur.dy) | non_finite(cur.dz);
         int k = 0;
-        double n2 = n1;
-        auto index_after = [&](int kk) {
-            return !USE_TABLE ? eval_index(P.mat[kk + 1], wl0)
-                              : (unlisted ? index_for_unlisted(&P.mat[kk + 1], wl0) : s_ntab[row + kk + 1]);
-        };
-        auto radius_rcp = [&](const DevSurface &s, int kk) {
-            xm::Rcp r;
-            r.b = (s.kind == RTB_SURF_PERFECT_LENS) ? s.focal_len : s.radius;
-            r.y = s_c.rcp_radius[kk];
-            r.ok = (s_c.rcp_ok >> kk) & 1ull;
-            return r;
-        };
-        // One surface with nothing to keep.  It runs optimistically; one flag says whether every intermediate stayed
-        // in the fast paths' domain, otherwise the surface is redone with the Careful arithmetic (surface_steps.cuh).
-        auto plain_surface = [&](int kk) {
-            const DevSurface &s = P.surf[kk];
-            n2 = index_after(kk);
-            const xm::Rcp rcp_k = radius_rcp(s, kk);
-            Optimistic m;
-            m.ok = !force_careful;
-            force_careful = false;
-            AtRaw raw;
-            Ray after;
-            if (s.kind == RTB_SURF_FLAT || s.kind == RTB_SURF_SPHERE) {
-                const double ratio = (USE_TABLE && !unlisted) ? s_ratio[row + kk] : xm::div(n1, n2);
-                dead = refracting_step<Optimistic, false>(m, s, cur, n1, ratio, rcp_wl, rcp_k, !intersect_only, raw,
-                                                          after);
-                if (!m.ok) {
-                    const StepResult redo = careful_refracting(&s, cur, n1, ratio, !intersect_only);
-                    after = redo.after;
-                    dead = redo.dead;
-                }
-            } else if (s.kind == RTB_SURF_MIRROR) {
-                dead = mirror_step<Optimistic, false>(m, s, cur, n1, rcp_wl, raw, after);
-                if (!m.ok) {
-                    const StepResult redo = careful_mirror(&s, cur, n1);
-                    after = redo.after;
-                    dead = redo.dead;
-                }
-            } else {
-                dead = perfect_lens_step<Optimistic>(m, s, cur, n1, n2, rcp_wl, rcp_k, intersect_only, false, raw, after);
-                if (!m.ok) {
-                    const StepResult redo = careful_lens(&s, cur, n1, n2, intersect_only);
-                    after = redo.after;
-                    dead = redo.dead;
-                }
-            }
-            cur = after;
-            n1 = n2;
-        };
         // act (uniform per surface): bit 0 store "at", 1 store "after", 2 reduce "at", 3 reduce "after"
         auto emit_after = [&](int kk, int act) {
-            Ray out = cur;
-            if (dead) set_nan(out); // the optimistic step leaves a culled ray's values un-blanked
+            Ray out = st.cur;
+            if (st.dead) set_nan(out); // the optimistic step leaves a culled ray's values un-blanked
             if (act & 2) store_ray(P.out + P.slab_pos[2 * kk + 2] * P.out_stride, row0 + i, out_rows, planes_out, out);
             if (act & 8) reduce_sample(red, out, tally);
         };
-        // One surface whose "at" slab is stored or reduced.
+        // One surface whose "at" slab is stored or reduced.  (Each kind's redo sits in its own branch, as in
+        // plain_surface_step: one careful_step after the branches costs the general kernel FP64 instructions and spills.)
         auto observed_surface = [&](int kk, int act) {
             const DevSurface &s = P.surf[kk];
-            n2 = index_after(kk);
-            const xm::Rcp rcp_k = radius_rcp(s, kk);
+            st.n2 = index_after<USE_TABLE>(P, s_ntab, kk, st);
+            const xm::Rcp rcp_k = radius_rcp(s, s_c, kk);
             const bool need_at = (act & 5) != 0;
             auto emit_at = [&](const Ray &at) {
                 if (act & 1) store_ray(P.out + P.slab_pos[2 * kk + 1] * P.out_stride, row0 + i, out_rows, planes_out, at);
                 if (act & 4) reduce_sample(red, at, tally);
             };
             Optimistic m;
-            m.ok = !force_careful;
-            force_careful = false;
+            m.ok = !st.force_careful;
+            st.force_careful = false;
             AtRaw raw;
             Ray after;
             if (s.kind == RTB_SURF_FLAT || s.kind == RTB_SURF_SPHERE) {
-                const double ratio = (USE_TABLE && !unlisted) ? s_ratio[row + kk] : xm::div(n1, n2);
-                dead = refracting_step<Optimistic, true>(m, s, cur, n1, ratio, rcp_wl, rcp_k, !intersect_only, raw,
-                                                         after);
+                const double ratio = (USE_TABLE && !st.unlisted) ? s_ratio[st.row + kk] : xm::div(st.n1, st.n2);
+                st.dead = refracting_step<Optimistic, true>(m, s, st.cur, st.n1, ratio, st.rcp_wl, rcp_k, !intersect_only,
+                                                            raw, after);
                 if (!m.ok) {
-                    const StepResult redo = careful_refracting(&s, cur, n1, ratio, !intersect_only);
+                    const StepResult redo = careful_refracting(&s, st.cur, st.n1, ratio, !intersect_only);
                     if (need_at) emit_at(redo.at);
                     after = redo.after;
-                    dead = redo.dead;
+                    st.dead = redo.dead;
                 }
             } else if (s.kind == RTB_SURF_MIRROR) {
-                dead = mirror_step<Optimistic, true>(m, s, cur, n1, rcp_wl, raw, after);
+                st.dead = mirror_step<Optimistic, true>(m, s, st.cur, st.n1, st.rcp_wl, raw, after);
                 if (!m.ok) {
-                    const StepResult redo = careful_mirror(&s, cur, n1);
+                    const StepResult redo = careful_mirror(&s, st.cur, st.n1);
                     if (need_at) emit_at(redo.at);
                     after = redo.after;
-                    dead = redo.dead;
+                    st.dead = redo.dead;
                 }
             } else {
-                dead = perfect_lens_step<Optimistic>(m, s, cur, n1, n2, rcp_wl, rcp_k, intersect_only, need_at, raw,
-                                                     after);
+                st.dead = perfect_lens_step<Optimistic>(m, s, st.cur, st.n1, st.n2, st.rcp_wl, rcp_k, intersect_only, need_at,
+                                                        raw, after);
                 if (!m.ok) {
-                    const StepResult redo = careful_lens(&s, cur, n1, n2, intersect_only);
+                    const StepResult redo = careful_lens(&s, st.cur, st.n1, st.n2, intersect_only);
                     if (need_at) emit_at(redo.at);
                     after = redo.after;
-                    dead = redo.dead;
+                    st.dead = redo.dead;
                 }
             }
             if (m.ok && need_at) {
                 Ray at;
-                fill_at(raw, cur, at);
+                fill_at(raw, st.cur, at);
                 emit_at(at);
             }
-            cur = after;
-            n1 = n2;
+            st.cur = after;
+            st.n1 = st.n2;
         };
         if (FINAL_RED) {
-            RayLoop st;
-            st.cur = cur;
-            st.n1 = n1;
-            st.n2 = n2;
-            st.wl0 = wl0;
-            st.rcp_wl = rcp_wl;
-            st.row = row;
-            st.unlisted = unlisted;
-            st.dead = false;
-            st.force_careful = force_careful;
             const int k_red = (P.red.slab - 2) >> 1;        // the sample is the slab after surface k_red
 #pragma unroll 1
-            for (; k <= k_red && !st.dead; k++) plain_surface_step<Optimistic, USE_TABLE>(P, s_ntab, s_ratio, s_c, k, st);
+            for (; k <= k_red && !st.dead; k++) plain_surface_step<Optimistic, USE_TABLE, false>(P, s_ntab, s_ratio, s_c, k, st);
             if (!st.dead) reduce_sample(red, st.cur, tally);
 #pragma unroll 1
-            for (; k < P.n_surf && !st.dead; k++) plain_surface_step<Optimistic, USE_TABLE>(P, s_ntab, s_ratio, s_c, k, st);
-            cur = st.cur;
-            dead = st.dead;
+            for (; k < P.n_surf && !st.dead; k++) plain_surface_step<Optimistic, USE_TABLE, false>(P, s_ntab, s_ratio, s_c, k, st);
         } else if (!GENERAL) {
             // two surfaces per trip: the ray's registers ping-pong between the two copies of the body instead of
             // being moved back at the end of every surface (+3 % here; the general mode's loop loses by it)
-            RayLoop st;
-            st.cur = cur;
-            st.n1 = n1;
-            st.n2 = n2;
-            st.wl0 = wl0;
-            st.rcp_wl = rcp_wl;
-            st.row = row;
-            st.unlisted = unlisted;
-            st.dead = false;
-            st.force_careful = force_careful;
             for (; k < P.n_surf && !st.dead; k += 2) {
-                plain_surface_step<Optimistic, USE_TABLE>(P, s_ntab, s_ratio, s_c, k, st);
-                if (k + 1 < P.n_surf && !st.dead) plain_surface_step<Optimistic, USE_TABLE>(P, s_ntab, s_ratio, s_c, k + 1, st);
+                plain_surface_step<Optimistic, USE_TABLE, false>(P, s_ntab, s_ratio, s_c, k, st);
+                if (k + 1 < P.n_surf && !st.dead) plain_surface_step<Optimistic, USE_TABLE, false>(P, s_ntab, s_ratio, s_c, k + 1, st);
             }
-            cur = st.cur;
-            dead = st.dead;
         } else {
             // runs of surfaces whose "at" slab is not needed go through the same tight loop as the final-slab-only kernel
-            while (k < P.n_surf && !dead) {
+            while (k < P.n_surf && !st.dead) {
 #pragma unroll 1
-                for (; k < P.n_surf && !dead && (P.slab_act[k] & 5) == 0; k++) {
-                    plain_surface(k);
+                for (; k < P.n_surf && !st.dead && (P.slab_act[k] & 5) == 0; k++) {
+                    plain_surface_step<Optimistic, USE_TABLE, intersect_only>(P, s_ntab, s_ratio, s_c, k, st);
                     const int act = P.slab_act[k];
                     if (act & 10) emit_after(k, act);
                 }
-                if (k < P.n_surf && !dead) {
+                if (k < P.n_surf && !st.dead) {
                     const int act = P.slab_act[k];
                     observed_surface(k, act);
                     if (act & 10) emit_after(k, act);
@@ -362,7 +301,7 @@ __global__ void __launch_bounds__(kTraceThreads, kTraceMinBlocks) trace_f64_kern
                 }
             }
         }
-        if (GENERAL && dead) {
+        if (GENERAL && st.dead) {
             // blank what is left of a dead ray's history (reductions skip NaN samples, nothing to add there)
             Ray blank;
             set_nan(blank);
@@ -374,8 +313,8 @@ __global__ void __launch_bounds__(kTraceThreads, kTraceMinBlocks) trace_f64_kern
             }
         }
         if (!GENERAL && (!FINAL_RED || P.any_store)) {
-            if (dead) set_nan(cur);
-            store_ray(P.out, i, out_rows, planes_out, cur);
+            if (st.dead) set_nan(st.cur);
+            store_ray(P.out, i, out_rows, planes_out, st.cur);
         }
     }
     if ((GENERAL || FINAL_RED) && reducing) tally_flush(red, tally);

@@ -253,11 +253,7 @@ __global__ void __launch_bounds__(128, sizeof(T) == 8 ? 4 : 6) trace_fast_kernel
         int row = 0;
         bool unlisted = false;
         if (USE_TABLE) {
-            row = P.n_wl;
-            const long long bits = __double_as_longlong(wl0);
-#pragma unroll 1
-            for (int q = 0; q < P.n_wl; q++)
-                if (__double_as_longlong(P.wl[q]) == bits) row = q;
+            row = wavelength_row(P, wl0);
             unlisted = (row == P.n_wl) && (wl0 == wl0);
             row *= n_med;
         }

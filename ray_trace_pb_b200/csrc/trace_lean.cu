@@ -88,10 +88,7 @@ static __device__ __noinline__ void redo_ray(const TraceParams *P, Ray cur, int 
     int row = 0;
     bool unlisted = false;
     if (USE_TABLE) {
-        row = P->n_wl;
-        const long long bits = __double_as_longlong(wl0);
-        for (int k = 0; k < P->n_wl; k++)
-            if (__double_as_longlong(P->wl[k]) == bits) row = k;
+        row = wavelength_row(*P, wl0);
         unlisted = (row == P->n_wl) && (wl0 == wl0);
         row *= n_med;
     }
@@ -108,15 +105,9 @@ static __device__ __noinline__ void redo_ray(const TraceParams *P, Ray cur, int 
         if (!dead) {
             const DevSurface *s = &P->surf[k];
             const double n2 = index_of(k + 1);
-            StepResult res;
-            if (s->kind == RTB_SURF_FLAT || s->kind == RTB_SURF_SPHERE) {
-                const double ratio = (USE_TABLE && !unlisted) ? P->ratio_tab[row + k] : xm::div(n1, n2);
-                res = careful_refracting(s, cur, n1, ratio, true);
-            } else if (s->kind == RTB_SURF_MIRROR) {
-                res = careful_mirror(s, cur, n1);
-            } else {
-                res = careful_lens(s, cur, n1, n2, false);
-            }
+            // (the ratio is only read at refracting surfaces)
+            const double ratio = (USE_TABLE && !unlisted) ? P->ratio_tab[row + k] : xm::div(n1, n2);
+            const StepResult res = careful_step(s, cur, n1, n2, ratio, false);
             if (k == k_sample && sample_at) *sample_row = res.at;
             cur = res.after;
             dead = res.dead;
@@ -230,6 +221,25 @@ __device__ __forceinline__ bool general_step(const DevSurface &s, int code, doub
     return !dead;
 }
 
+// the step of surface s by its code: the probe-driven kernels' runs of mixed codes, and the probe
+template <int KINDS>
+__device__ __forceinline__ bool surface_step(const DevSurface &s, SurfaceShared ss, lean::State &r, double n1,
+                                             double n2, double ratio, double wl0, double wl_rcp, const double2 *near_one,
+                                             bool &ok, bool &kill)
+{
+    if (ss.code == kLeanSphere) return lean::sphere_axial(ok, s, ss.rcp, r, n1, ratio, wl0, wl_rcp, near_one, kill);
+    if (ss.code == kLeanFlat) return lean::flat_axial<false>(ok, s, r, n1, ratio, wl0, wl_rcp, near_one, kill);
+    if (ss.code == kLeanFlatZ) return lean::flat_axial<true>(ok, s, r, n1, ratio, wl0, wl_rcp, near_one, kill);
+    if (KINDS == 1 && ss.code == kLeanFlatAny) return lean::flat_any(ok, s, r, n1, ratio, wl0, wl_rcp, near_one, kill);
+    if (KINDS == 1 && ss.code == kLeanLens) {
+        kill = true;       // (a perfect lens's "at" slab is not offered as a sample: lean_eligible)
+        return lean::lens_any(ok, s, ss.rcp, r, n1, n2, wl0, wl_rcp);
+    }
+    // (KINDS = 0: the launcher has made sure that only refracting surfaces get here)
+    return general_step(s, KINDS == 1 ? ss.code : (int)kGeneralRefracting, ss.rcp, ss.rcp_ok != 0, r, n1, n2, ratio, wl0,
+                        wl_rcp, ok, kill);
+}
+
 // ---- the kernel --------------------------------------------------------------------------------------------------
 // USE_TABLE / FROM_SOURCE as in trace_f64.cu.  SWEEP: blockIdx.y picks the source, its output rows and its reduction
 // bucket (rtb_trace_sources).  PROBE: the probe launch -- a strided sample of the rays, per-surface recovery, counts only.
@@ -270,7 +280,7 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
         const DevSurface &s = P.surf[k];
         const double den = (s.kind == RTB_SURF_PERFECT_LENS) ? s.focal_len : s.radius;
         const double rcp = xm::refine_rcp(den);
-        const bool sane = xm::den_ok(den) && fabs(den) < 4503599627370496.0 && xm::quo_ok(rcp);
+        const bool sane = usable_rcp(den, rcp);
         s_c.surf[k].rcp = rcp;
         s_c.surf[k].rcp_ok = sane;
         // a sphere / lens whose reciprocal radius / focal length is unusable goes through the general step (which flags
@@ -324,20 +334,11 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
         }
         const double wl0 = cur.wl;
         const double wl_rcp = xm::refine_rcp(wl0);
-        int row = 0;
-        bool listed = true;
-        if (USE_TABLE) {
-            row = P.n_wl;
-            const long long bits = __double_as_longlong(wl0);
-#pragma unroll 1
-            for (int k = 0; k < P.n_wl; k++)
-                if (__double_as_longlong(P.wl[k]) == bits) row = k;
-            listed = row != P.n_wl;              // NaN and unlisted wavelengths take the careful route
-        }
+        const int row = USE_TABLE ? wavelength_row(P, wl0) : 0;
+        const bool listed = !USE_TABLE || row != P.n_wl;   // NaN and unlisted wavelengths take the careful route
         const double *pair = s_pair + 2 * row * n_med;
         // The lean and optimistic steps assume finite geometry and a wavelength in [2^-100, 2^100] (then no phase
         // quotient can leave the normal range); anything else is the careful route's business.
-        auto non_finite = [](double v) { return (__double2hiint(v) & 0x7ff00000) == 0x7ff00000; };
         const unsigned wl_exp = ((unsigned)__double2hiint(wl0) >> 20) & 0x7ffu;
         const bool fit = valid && listed && (wl_exp - 923u <= 200u) &&
                          !(non_finite(cur.ox) | non_finite(cur.oy) | non_finite(cur.oz) | non_finite(cur.dx) |
@@ -356,6 +357,32 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
             // uniform datapath / constant bank instead of vector registers.  Whole warps of dead rays leave early.
             // (each run's loop has its own induction variable, defined from kernel parameters only: the general steps
             // branch on values loaded through theirs, which makes it a vector register; the lean loops' stay uniform)
+            // One run of surfaces that take the same step: step(k, n2, ratio, ok, kill) advances the ray through surface k
+            // and returns whether it is still on (a step that does not read n2 or the ratio leaves their fetch dead)
+            auto run_surfaces = [&](int begin, int end, auto step) {
+                for (int k = begin; k < end; k++) {
+                    if (!__any_sync(0xffffffffu, alive)) {
+                        at_valid = false;      // (the surface that would have been sampled is not reached)
+                        break;
+                    }
+                    double ratio, n2;
+                    if (USE_TABLE) {
+                        n1 = pair[0];
+                        ratio = pair[1];
+                        n2 = pair[2];
+                        pair += 2;
+                    } else {
+                        n2 = eval_index(P.mat[k + 1], wl0);
+                        ratio = xm::div(n1, n2);
+                    }
+                    bool ok = true, kill;
+                    const bool on = step(k, n2, ratio, ok, kill);
+                    failed = failed | (alive & !ok);
+                    at_valid = alive & ok & !kill;
+                    alive = alive & ok & on;
+                    if (!USE_TABLE) n1 = n2;
+                }
+            };
             for (int run = 0; run < P.lean_n_runs; run++) {
                 const int begin = run > 0 ? P.lean_run_end[run - 1] : 0;
                 const int end = P.lean_run_end[run];
@@ -363,197 +390,48 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
                 // (an overridden run goes through the loop that dispatches per surface)
                 const int code = (KINDS >= 2 || s_c.run_clean[run]) ? P.lean_run_code[run] : kMixedRun;
                 if (code == kLeanSphere) {
-                    for (int k = begin; k < end; k++) {
-                        if (!__any_sync(0xffffffffu, alive)) {
-                            at_valid = false;      // (the surface that would have been sampled is not reached)
-                            break;
-                        }
-                        if (USE_TABLE) {
-                            n1 = pair[0];
-                            pair += 2;
-                        }
-                        const double n2 = USE_TABLE ? 0.0 : eval_index(P.mat[k + 1], wl0);
-                        const double ratio = USE_TABLE ? pair[-1] : xm::div(n1, n2);
-                        bool ok = true, kill;
-                        const bool on = lean::sphere_axial(ok, P.surf[k], s_c.surf[k].rcp, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                        failed = failed | (alive & !ok);
-                        at_valid = alive & ok & !kill;
-                        alive = alive & ok & on;
-                        if (!USE_TABLE) n1 = n2;
-                    }
+                    run_surfaces(begin, end, [&](int k, double, double ratio, bool &ok, bool &kill) {
+                        return lean::sphere_axial(ok, P.surf[k], s_c.surf[k].rcp, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
+                    });
                 } else if (code == kLeanFlat) {
-                    for (int k = begin; k < end; k++) {
-                        if (!__any_sync(0xffffffffu, alive)) {
-                            at_valid = false;      // (the surface that would have been sampled is not reached)
-                            break;
-                        }
-                        if (USE_TABLE) {
-                            n1 = pair[0];
-                            pair += 2;
-                        }
-                        const double n2 = USE_TABLE ? 0.0 : eval_index(P.mat[k + 1], wl0);
-                        const double ratio = USE_TABLE ? pair[-1] : xm::div(n1, n2);
-                        bool ok = true, kill;
-                        const bool on = lean::flat_axial<false>(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                        failed = failed | (alive & !ok);
-                        at_valid = alive & ok & !kill;
-                        alive = alive & ok & on;
-                        if (!USE_TABLE) n1 = n2;
-                    }
+                    run_surfaces(begin, end, [&](int k, double, double ratio, bool &ok, bool &kill) {
+                        return lean::flat_axial<false>(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
+                    });
                 } else if (KINDS >= 2 && code == kLeanFlatZ) {
                     // (pure kernels only: the zero-tolerant on-axis flat where the cached verdict asks for it; the
                     // probe-driven kernels reach this step through their dispatching loop)
-                    for (int k = begin; k < end; k++) {
-                        if (!__any_sync(0xffffffffu, alive)) {
-                            at_valid = false;
-                            break;
-                        }
-                        if (USE_TABLE) {
-                            n1 = pair[0];
-                            pair += 2;
-                        }
-                        const double n2 = USE_TABLE ? 0.0 : eval_index(P.mat[k + 1], wl0);
-                        const double ratio = USE_TABLE ? pair[-1] : xm::div(n1, n2);
-                        bool ok = true, kill;
-                        const bool on = lean::flat_axial<true>(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                        failed = failed | (alive & !ok);
-                        at_valid = alive & ok & !kill;
-                        alive = alive & ok & on;
-                        if (!USE_TABLE) n1 = n2;
-                    }
+                    run_surfaces(begin, end, [&](int k, double, double ratio, bool &ok, bool &kill) {
+                        return lean::flat_axial<true>(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
+                    });
                 } else if ((KINDS == 1 || KINDS == 3) && code == kLeanFlatAny) {
-                    for (int k = begin; k < end; k++) {
-                        if (!__any_sync(0xffffffffu, alive)) {
-                            at_valid = false;
-                            break;
-                        }
-                        if (USE_TABLE) {
-                            n1 = pair[0];
-                            pair += 2;
-                        }
-                        const double n2 = USE_TABLE ? 0.0 : eval_index(P.mat[k + 1], wl0);
-                        const double ratio = USE_TABLE ? pair[-1] : xm::div(n1, n2);
-                        bool ok = true, kill;
-                        const bool on = lean::flat_any(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                        failed = failed | (alive & !ok);
-                        at_valid = alive & ok & !kill;
-                        alive = alive & ok & on;
-                        if (!USE_TABLE) n1 = n2;
-                    }
+                    run_surfaces(begin, end, [&](int k, double, double ratio, bool &ok, bool &kill) {
+                        return lean::flat_any(ok, P.surf[k], r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
+                    });
                 } else if ((KINDS == 1 || KINDS == 3) && code == kLeanLens) {
-                    for (int k = begin; k < end; k++) {
-                        if (!__any_sync(0xffffffffu, alive)) {
-                            at_valid = false;
-                            break;
-                        }
-                        double n2;
-                        if (USE_TABLE) {
-                            n1 = pair[0];
-                            n2 = pair[2];
-                            pair += 2;
-                        } else {
-                            n2 = eval_index(P.mat[k + 1], wl0);
-                        }
-                        bool ok = true;
-                        const bool on = lean::lens_any(ok, P.surf[k], s_c.surf[k].rcp, r, n1, n2, wl0, wl_rcp);
-                        failed = failed | (alive & !ok);
-                        at_valid = false;
-                        alive = alive & ok & on;
-                        if (!USE_TABLE) n1 = n2;
-                    }
+                    run_surfaces(begin, end, [&](int k, double n2, double, bool &ok, bool &kill) {
+                        kill = true;       // (a perfect lens's "at" slab is not offered as a sample: lean_eligible)
+                        return lean::lens_any(ok, P.surf[k], s_c.surf[k].rcp, r, n1, n2, wl0, wl_rcp);
+                    });
                 } else if (KINDS == 1 && code == kGeneralLens) {
                     // a run of perfect lenses: its own loop, so that the hot code of a lens train (the OPM: 4f relays of
                     // perfect lenses and flats) is this step and the flats' -- not every step the kernel knows
-                    for (int k = begin; k < end; k++) {
-                        if (!__any_sync(0xffffffffu, alive)) {
-                            at_valid = false;
-                            break;
-                        }
-                        const DevSurface &s = P.surf[k];
+                    run_surfaces(begin, end, [&](int k, double n2, double ratio, bool &ok, bool &kill) {
                         const SurfaceShared ss = s_c.surf[k];
-                        double ratio, n2;
-                        if (USE_TABLE) {
-                            n1 = pair[0];
-                            ratio = pair[1];
-                            n2 = pair[2];
-                            pair += 2;
-                        } else {
-                            n2 = eval_index(P.mat[k + 1], wl0);
-                            ratio = xm::div(n1, n2);
-                        }
-                        bool ok = true, kill;
-                        const bool on = general_step(s, kGeneralLens, ss.rcp, ss.rcp_ok != 0, r, n1, n2, ratio, wl0, wl_rcp, ok, kill);
-                        failed = failed | (alive & !ok);
-                        at_valid = alive & ok & !kill;
-                        alive = alive & ok & on;
-                        if (!USE_TABLE) n1 = n2;
-                    }
+                        return general_step(P.surf[k], kGeneralLens, ss.rcp, ss.rcp_ok != 0, r, n1, n2, ratio, wl0, wl_rcp,
+                                            ok, kill);
+                    });
                 } else if (KINDS < 2 && code == kGeneralRefracting) {
                     // tilted / decentred flats and spheres, or ones the launcher keeps off the lean steps
-                    for (int k = begin; k < end; k++) {
-                        if (!__any_sync(0xffffffffu, alive)) {
-                            at_valid = false;
-                            break;
-                        }
-                        const DevSurface &s = P.surf[k];
+                    run_surfaces(begin, end, [&](int k, double n2, double ratio, bool &ok, bool &kill) {
                         const SurfaceShared ss = s_c.surf[k];
-                        double ratio, n2 = 0.0;
-                        if (USE_TABLE) {
-                            n1 = pair[0];
-                            ratio = pair[1];
-                            pair += 2;
-                        } else {
-                            n2 = eval_index(P.mat[k + 1], wl0);
-                            ratio = xm::div(n1, n2);
-                        }
-                        bool ok = true, kill;
-                        const bool on = general_step(s, kGeneralRefracting, ss.rcp, ss.rcp_ok != 0, r, n1, n2, ratio, wl0, wl_rcp, ok, kill);
-                        failed = failed | (alive & !ok);
-                        at_valid = alive & ok & !kill;
-                        alive = alive & ok & on;
-                        if (!USE_TABLE) n1 = n2;
-                    }
+                        return general_step(P.surf[k], kGeneralRefracting, ss.rcp, ss.rcp_ok != 0, r, n1, n2, ratio, wl0,
+                                            wl_rcp, ok, kill);
+                    });
                 } else if (KINDS < 2) {
-                    for (int k = begin; k < end; k++) {
-                        if (!__any_sync(0xffffffffu, alive)) {
-                            at_valid = false;      // (the surface that would have been sampled is not reached)
-                            break;
-                        }
-                        const DevSurface &s = P.surf[k];
-                        const SurfaceShared ss = s_c.surf[k];
-                        double ratio, n2 = 0.0;
-                        if (USE_TABLE) {
-                            n1 = pair[0];
-                            ratio = pair[1];
-                            n2 = pair[2];
-                            pair += 2;
-                        } else {
-                            n2 = eval_index(P.mat[k + 1], wl0);
-                            ratio = xm::div(n1, n2);
-                        }
-                        bool ok = true, kill;
-                        bool on;
-                        if (ss.code == kLeanSphere) {
-                            on = lean::sphere_axial(ok, s, ss.rcp, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                        } else if (ss.code == kLeanFlat) {
-                            on = lean::flat_axial<false>(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                        } else if (ss.code == kLeanFlatZ) {
-                            on = lean::flat_axial<true>(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                        } else if (KINDS == 1 && ss.code == kLeanFlatAny) {
-                            on = lean::flat_any(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                        } else if (KINDS == 1 && ss.code == kLeanLens) {
-                            on = lean::lens_any(ok, s, ss.rcp, r, n1, n2, wl0, wl_rcp);
-                            kill = false;
-                        } else {
-                            // (KINDS = 0: the launcher has made sure that only refracting surfaces get here)
-                            on = general_step(s, KINDS == 1 ? ss.code : (int)kGeneralRefracting, ss.rcp, ss.rcp_ok != 0, r, n1,
-                                              n2, ratio, wl0, wl_rcp, ok, kill);
-                        }
-                        failed = failed | (alive & !ok);
-                        at_valid = alive & ok & !kill;
-                        alive = alive & ok & on;
-                        if (!USE_TABLE) n1 = n2;
-                    }
+                    run_surfaces(begin, end, [&](int k, double n2, double ratio, bool &ok, bool &kill) {
+                        return surface_step<KINDS>(P.surf[k], s_c.surf[k], r, n1, n2, ratio, wl0, wl_rcp, s_c.near_one, ok,
+                                                   kill);
+                    });
                 }
                 // the sample: the slab after the run's last surface, or (odd slab) the one at it -- whose position and
                 // phase the step has left in the ray, valid unless the ray was culled there
@@ -567,8 +445,6 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
             for (int k = 0; k < P.n_surf; k++) {
                 if (!alive) break;
                 const DevSurface &s = P.surf[k];
-                const SurfaceShared ss = s_c.surf[k];
-                const int code = ss.code;
                 double ratio, n2;
                 if (USE_TABLE) {
                     n1 = pair[0];
@@ -580,19 +456,8 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
                     ratio = xm::div(n1, n2);
                 }
                 const lean::State before = r;
-                bool ok = true, on, kill;
-                if (code == kLeanSphere)
-                    on = lean::sphere_axial(ok, s, ss.rcp, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                else if (code == kLeanFlat)
-                    on = lean::flat_axial<false>(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                else if (code == kLeanFlatZ)
-                    on = lean::flat_axial<true>(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                else if (code == kLeanFlatAny)
-                    on = lean::flat_any(ok, s, r, n1, ratio, wl0, wl_rcp, s_c.near_one, kill);
-                else if (code == kLeanLens)
-                    on = lean::lens_any(ok, s, ss.rcp, r, n1, n2, wl0, wl_rcp);
-                else
-                    on = general_step(s, code, ss.rcp, ss.rcp_ok != 0, r, n1, n2, ratio, wl0, wl_rcp, ok, kill);
+                bool ok = true, kill;
+                bool on = surface_step<1>(s, s_c.surf[k], r, n1, n2, ratio, wl0, wl_rcp, s_c.near_one, ok, kill);  // (every kind)
                 atomicAdd(my_counts + 2 * k, 1u);
                 if (!ok) {
                     atomicAdd(my_counts + 2 * k + 1, 1u);
@@ -600,13 +465,7 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
                     in.ox = before.ox; in.oy = before.oy; in.oz = before.oz;
                     in.dx = before.dx; in.dy = before.dy; in.dz = before.dz;
                     in.ph = before.ph; in.wl = wl0;
-                    StepResult res;
-                    if (s.kind == RTB_SURF_FLAT || s.kind == RTB_SURF_SPHERE)
-                        res = careful_refracting(&s, in, n1, ratio, true);
-                    else if (s.kind == RTB_SURF_MIRROR)
-                        res = careful_mirror(&s, in, n1);
-                    else
-                        res = careful_lens(&s, in, n1, n2, false);
+                    const StepResult res = careful_step(&s, in, n1, n2, ratio, false);
                     r.ox = res.after.ox; r.oy = res.after.oy; r.oz = res.after.oz;
                     r.dx = res.after.dx; r.dy = res.after.dy; r.dz = res.after.dz;
                     r.ph = res.after.ph;
