@@ -229,7 +229,8 @@ int64_t rtb_launch_count(void);
 int64_t rtb_pure_launch_count(void);
 
 /*
- * Tuning knobs (never change a result, only which kernel gets there):
+ * Tuning knobs (never change a result, only which kernel gets there).  The environment variables named below set
+ * initial values; they are read when the library is loaded, and rtb_tune overrides them.
  *   "lean_min_rays"  launches of at least this many rays that keep only the final slab and / or one after-surface
  *                    reduction run the probe + lean kernel pair (csrc/trace_lean.cu); default 32768, negative = never.
  *                    The environment variable RTB_LEAN_MIN_RAYS sets the initial value.

@@ -21,10 +21,6 @@
 
 #include "rtb_device.cuh"
 
-namespace rtb {
-int api_fail(int code, const char *fmt, ...);      // rtb_api.cu: sets rtb_last_error
-}
-
 namespace {
 
 struct NcclApi {

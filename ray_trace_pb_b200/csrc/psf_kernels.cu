@@ -10,12 +10,16 @@
 // image coordinate = lambda f fx).  A "zoomed DFT": any sampling and window, no padding; for odd G, M = G and
 // df = 1/(G*cell) it is exactly fftshift(fft2(ifftshift(P))) (odd M puts a sample on the zero frequency).
 // fp64 throughout: tcgen05 has no f64 kind, so this runs on the FP64 pipe (64x64 register-tiled, K-split complex GEMM).
+#include <atomic>
 #include <cmath>
 #include <math_constants.h>
 
 #include "rtb_device.cuh"
 
 namespace rtb {
+
+// which contraction kernel runs: 1 = DMMA (mma.sync.m8n8k4.f64), 0 = the SIMT register-tiled one (rtb_tune "psf_dmma")
+std::atomic<long long> g_psf_dmma{1};
 
 namespace {
 
@@ -219,9 +223,6 @@ __global__ void abs2_kernel(const double *__restrict__ re, const double *__restr
         out[i] = fma(re[i], re[i], im[i] * im[i]);
 }
 
-// which contraction kernel runs: 1 = DMMA (mma.sync.m8n8k4.f64), 0 = the SIMT register-tiled one (rtb_tune "psf_dmma")
-int g_psf_dmma = 1;
-
 // K split so that the grid is at least ~4 waves of blocks (each block still loops over >= 4 k-steps)
 int zgemm_split(int Mx, int Ny, int K, int sm_count, int *k_chunk_out)
 {
@@ -242,7 +243,7 @@ cudaError_t launch_zgemm(int Mx, int Ny, int K, const double *x_re, const double
     const int split = zgemm_split(Mx, Ny, K, sm_count, &k_chunk);
     dim3 grid((Ny + kTile - 1) / kTile, (Mx + kTile - 1) / kTile, split);
     const long long n = (long long)Mx * Ny;
-    const bool tensor = g_psf_dmma != 0;
+    const bool tensor = g_psf_dmma.load(std::memory_order_relaxed) != 0;
     if (split == 1) {
         if (tensor)
             zgemm_nt_dmma_kernel<<<grid, 256, 0, stream>>>(Mx, Ny, K, k_chunk, x_re, x_im, y_re, y_im, c_re, c_im);
@@ -261,8 +262,6 @@ cudaError_t launch_zgemm(int Mx, int Ny, int K, const double *x_re, const double
 }
 
 } // namespace
-
-void set_psf_dmma(int on) { g_psf_dmma = on; }
 
 // scratch layout (doubles): [0, 2MG) DFT matrix D (re, im) ; [2MG, 4MG) Wt (re, im) ; [4MG, 4MG + 2MM) the field E when
 // the caller does not take it ; then 2GG for the normalised pupil ; then the K-split partial sums of the larger product

@@ -2,6 +2,7 @@
 // pinned-memory host pipeline.  No ray arithmetic happens here and nothing here runs a trace on the CPU.
 #include <algorithm>
 #include <atomic>
+#include <climits>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -16,13 +17,11 @@
 namespace rtb {
 cudaError_t launch_trace_f64(const TraceParams &P, int sm_count, cudaStream_t stream);
 cudaError_t launch_trace_fast(const TraceParams &P, int precision, int sm_count, cudaStream_t stream);
-bool lean_eligible(const TraceParams &P);
-void set_lean_min_share_pct(int pct);
-void set_psf_dmma(int on);
-cudaError_t launch_trace_lean(const TraceParams &P, unsigned *counts, int sm_count, cudaStream_t stream, int *launches,
-                              int pure_mode, unsigned long long verdict_general, bool *pure_used, bool probe_optional,
-                              bool *probed);
-unsigned long long lean_verdict_from_counts(const unsigned *counts, int n_src, int n_surf);
+bool lean_takes(const TraceParams &P, int precision);
+size_t lean_scratch_bytes(int n_sources);
+cudaError_t launch_lean(const TraceParams &P, int device, int sm_count, cudaStream_t stream, cudaMemPool_t pool,
+                        void *scratch, const DevSource *sources, int *launches);
+void lean_forget_verdicts();
 cudaError_t launch_generate(const DevSource &src, long long n_rays, double *out, int sm_count, cudaStream_t stream);
 cudaError_t launch_reduce_init(const DevReduce &red, int sm_count, cudaStream_t stream);
 cudaError_t launch_intersect(const double *r1, long long n1, const double *r2, long long n2, double *out,
@@ -39,27 +38,17 @@ cudaError_t run_exact_math_selftest(unsigned long long seed, long long n, unsign
 cudaError_t run_dfma_probe(int sm_count, double *dfma_per_s, double *elapsed_ms);
 cudaError_t run_dfma_chain_probe(int sm_count, int chains, double *dfma_per_s, double *elapsed_ms);
 cudaError_t run_copy_probe(long long bytes, double *bytes_per_s);
+// the tuning knobs of trace_lean.cu and psf_kernels.cu
+extern std::atomic<long long> g_lean_min_rays, g_lean_min_share_pct, g_lean_pure, g_keep_probe_counts, g_psf_dmma;
 } // namespace rtb
 
 namespace {
 
 thread_local char g_err[512] = "";
 std::atomic<long long> g_launches{0};
-// launches of at least this many rays that keep only the final slab / one reduction go to the lean kernel (probe launch
-// + trace launch, trace_lean.cu); smaller ones are not worth a probe.  rtb_tune("lean_min_rays", n); negative = never.
-std::atomic<long long> g_lean_min_rays{32768};
 // test hook: rtb_trace_host fails (RTB_ERR_CUDA, "injected") when it is about to launch chunk number n (0-based) of a
 // call; negative = off.  rtb_tune("host_fail_chunk", n).  Lets the tests check that an error return leaves no copy in flight.
 std::atomic<long long> g_host_fail_chunk{-1};
-// test hook: rtb_tune("keep_probe_counts", 1) makes every lean launch synchronise and keep its probe's counts (first
-// source only) for rtb_last_probe_counts()
-std::atomic<long long> g_keep_probe_counts{0};
-unsigned g_last_probe_counts[2 * RTB_MAX_SURFACES];
-// rtb_tune("lean_pure", m): 0 = the probe-driven lean kernels only; 1 (default) = the pure lean kernels once an earlier
-// probe of the same system and bundle has said that every surface can run its lean step (the verdict cache below);
-// 2 = the pure kernels whenever the system has a lean step for every surface, whatever the bundle (tests).
-std::atomic<long long> g_lean_pure{1};
-std::atomic<long long> g_pure_launches{0};
 // rtb_trace_sources traces sweeps of at least this many rays per source as one launch PER SOURCE (each with its source and
 // its reduction bucket in the kernel parameters, i.e. warp-uniform operands) instead of one launch whose blocks fetch
 // theirs from shared memory.  Measured: 3 x 16.8 M rays +3.6 % (BASELINE config 2: 65.3 -> 67.7 G ray*surf/s), but
@@ -67,19 +56,36 @@ std::atomic<long long> g_pure_launches{0};
 // split.  rtb_tune("sweep_split_rays", n); RTB_SWEEP_SPLIT_RAYS; negative = never.
 std::atomic<long long> g_sweep_split_rays{1 << 24};
 
-int fail(int code, const char *fmt, ...)
-{
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_err, sizeof(g_err), fmt, ap);
-    va_end(ap);
-    return code;
-}
+// rtb_tune's keys (include/rtb.h): the knob each sets, the environment variable that sets its initial value, and the
+// values it takes
+struct Knob {
+    const char *key;
+    const char *env;                  // (NULL: none)
+    std::atomic<long long> *value;
+    long long lo = LLONG_MIN, hi = LLONG_MAX;
+};
+const Knob kKnobs[] = {
+    {"lean_min_rays", "RTB_LEAN_MIN_RAYS", &rtb::g_lean_min_rays},
+    {"lean_min_share_pct", "RTB_LEAN_MIN_SHARE_PCT", &rtb::g_lean_min_share_pct},
+    {"lean_pure", "RTB_LEAN_PURE", &rtb::g_lean_pure, 0, 2},
+    {"psf_dmma", nullptr, &rtb::g_psf_dmma},
+    {"sweep_split_rays", "RTB_SWEEP_SPLIT_RAYS", &g_sweep_split_rays},
+    {"keep_probe_counts", nullptr, &rtb::g_keep_probe_counts},
+    {"host_fail_chunk", nullptr, &g_host_fail_chunk},
+};
+
+// The environment is read when the library is loaded, before any rtb_tune call, which therefore always wins.  (An
+// environment value outside the knob's range is clamped.)
+const bool g_knobs_from_env = [] {
+    for (const Knob &k : kKnobs)
+        if (const char *env = k.env ? getenv(k.env) : nullptr)
+            k.value->store(std::min(k.hi, std::max(k.lo, (long long)atoll(env))), std::memory_order_relaxed);
+    return true;
+}();
 
 } // namespace
 
 namespace rtb {
-// the same for the other translation units of the C ABI (comm.cu)
 int api_fail(int code, const char *fmt, ...)
 {
     va_list ap;
@@ -91,6 +97,17 @@ int api_fail(int code, const char *fmt, ...)
 } // namespace rtb
 
 namespace {
+
+constexpr auto &fail = rtb::api_fail;
+
+// The tail of an entry point that ran a launcher: RTB_ERR_CUDA ("<what>: <CUDA error>") if the launcher failed, else
+// its `n_kernels` kernels join rtb_launch_count().
+int launched(cudaError_t e, const char *what, long long n_kernels)
+{
+    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "%s: %s", what, cudaGetErrorString(e));
+    g_launches.fetch_add(n_kernels, std::memory_order_relaxed);
+    return RTB_OK;
+}
 
 #define RTB_CUDA(call)                                                                                     \
     do {                                                                                                   \
@@ -106,7 +123,7 @@ struct Slot {
     cudaStream_t stream = nullptr;
     cudaEvent_t done = nullptr;
     cudaEvent_t copied_in = nullptr;   // this slot's copy-in has landed (the previous chunk's copy-out waits for it)
-    unsigned *lean_counts = nullptr;   // probe scratch of the lean kernel for this slot's chunks
+    void *lean_scratch = nullptr;      // probe scratch of the lean kernel for this slot's chunks
     double *dev_in = nullptr;
     double *dev_out = nullptr;
     double *pin_in = nullptr;
@@ -114,47 +131,20 @@ struct Slot {
     size_t dev_in_bytes = 0, dev_out_bytes = 0, pin_in_bytes = 0, pin_out_bytes = 0;
 };
 
-// ---- the lean kernel's verdict cache (trace_lean.cu, DESIGN.md 4a) -------------------------------------------------
-// The pure instantiations of the lean kernel branch on kernel parameters only, so the choice "can every surface of this
-// system run its lean step with this bundle" has to be made on the host before the launch -- but the probe's counts are
-// on the device.  Every lean launch therefore copies its probe's counts to a pinned slot asynchronously (no
-// synchronisation), and the NEXT launch of the same system + bundle description picks its kernel by them.  A wrong verdict
-// costs time, never a bit of the result: rays that fail a lean step are re-traced by redo_ray in every kernel.  A key
-// whose verdict keeps changing (one system traced alternately with bundles of different character from device arrays)
-// stays with the probe-driven kernels.
-constexpr int kVerdictEntries = 128;
-constexpr int kVerdictMaxSources = 64;
-
-struct VerdictEntry {
-    unsigned long long key = 0;
-    bool used = false, have = false, pending = false;
-    unsigned long long general = 0;   // the last consumed probe's verdict (lean_verdict_from_counts)
-    int flips = 0, stable = 0;
-    int pending_n_src = 0, pending_n_surf = 0;
-    unsigned *pin = nullptr;          // pin_sources x kMaxSurfaces x 2 counts, page-locked
-    int pin_sources = 0;
-    cudaEvent_t ev = nullptr;
-    unsigned long long stamp = 0;
-};
-
 struct DeviceCtx {
     bool ready = false;
     int sm_count = 0;
     Slot slot[kSlots];
-    std::mutex verdict_mutex;
-    VerdictEntry verdict[kVerdictEntries];
-    unsigned long long verdict_clock = 0;
     std::mutex host_path; // one host-buffer trace at a time per device
     cudaMemPool_t pool = nullptr; // small stream-ordered allocations (sweep source lists); keeps its memory
 };
 
-constexpr int kMaxDevices = 64;
-DeviceCtx g_ctx[kMaxDevices];
+DeviceCtx g_ctx[rtb::kMaxDevices];
 std::mutex g_ctx_mutex;
 
 int get_ctx(int device, DeviceCtx **out)
 {
-    if (device < 0 || device >= kMaxDevices) return fail(RTB_ERR_INVALID, "device index %d out of range", device);
+    if (device < 0 || device >= rtb::kMaxDevices) return fail(RTB_ERR_INVALID, "device index %d out of range", device);
     int n = 0;
     cudaError_t e = cudaGetDeviceCount(&n);
     if (e != cudaSuccess || n == 0)
@@ -171,11 +161,16 @@ int get_ctx(int device, DeviceCtx **out)
     return RTB_OK;
 }
 
-struct DeviceGuard {
-    int prev = -1;
+// The device of an entry point: its context, and the device made current for the rest of the call (the caller's
+// current device comes back when this goes out of scope).
+struct OnDevice {
+    DeviceCtx *ctx = nullptr;
+    int device = -1, prev = -1;
     bool changed = false;
-    int enter(int device)
+    int enter(int dev)
     {
+        if (int rc = get_ctx(dev, &ctx)) return rc;
+        device = dev;
         RTB_CUDA(cudaGetDevice(&prev));
         if (prev != device) {
             RTB_CUDA(cudaSetDevice(device));
@@ -183,7 +178,7 @@ struct DeviceGuard {
         }
         return RTB_OK;
     }
-    ~DeviceGuard()
+    ~OnDevice()
     {
         if (changed) cudaSetDevice(prev);
     }
@@ -437,201 +432,25 @@ int ensure_pool(DeviceCtx *ctx, int device)
     return RTB_OK;
 }
 
-bool wants_lean(const rtb::TraceParams &P, int precision)
+// `lean_scratch`: the lean kernel's probe scratch, owned by the caller (the host pipeline's slots), or NULL to take it from
+// the device's stream-ordered pool for the duration of this launch.  `sources`: the host copy of the source
+// description(s) of a launch from on-device sources (the lean kernel's verdict cache keys on them).
+int launch(const rtb::TraceParams &P, int precision, const OnDevice &on, cudaStream_t stream,
+           void *lean_scratch = nullptr, const rtb::DevSource *sources = nullptr)
 {
-    static const bool env_read = [] {
-        if (const char *env = getenv("RTB_LEAN_MIN_RAYS")) g_lean_min_rays.store(atoll(env), std::memory_order_relaxed);
-        if (const char *env = getenv("RTB_LEAN_MIN_SHARE_PCT")) rtb::set_lean_min_share_pct(atoi(env));
-        if (const char *env = getenv("RTB_LEAN_PURE")) g_lean_pure.store(std::min(2ll, std::max(0ll, atoll(env))), std::memory_order_relaxed);
-        if (const char *env = getenv("RTB_SWEEP_SPLIT_RAYS")) g_sweep_split_rays.store(atoll(env), std::memory_order_relaxed);
-        return true;
-    }();
-    (void)env_read;
-    const long long min_rays = g_lean_min_rays.load(std::memory_order_relaxed);
-    return precision == RTB_F64_EXACT && min_rays >= 0 && P.n_rays >= min_rays && rtb::lean_eligible(P);
-}
-
-// 64-bit mix of a byte range (8 bytes at a time; the tail byte-wise)
-unsigned long long hash_bytes(unsigned long long h, const void *data, size_t n)
-{
-    const unsigned char *p = (const unsigned char *)data;
-    for (; n >= 8; n -= 8, p += 8) {
-        unsigned long long w;
-        memcpy(&w, p, 8);
-        h = (h ^ w) * 0x9E3779B97F4A7C15ull;
-        h ^= h >> 29;
+    DeviceCtx *ctx = on.ctx;
+    if (rtb::lean_takes(P, precision)) {
+        int rc, launches = 0;
+        if (!lean_scratch && (rc = ensure_pool(ctx, on.device))) return rc;
+        const cudaError_t e = rtb::launch_lean(P, on.device, ctx->sm_count, stream, lean_scratch ? nullptr : ctx->pool,
+                                               lean_scratch, sources, &launches);
+        if (e == cudaErrorMemoryAllocation)
+            return fail(RTB_ERR_NOMEM, "stream-ordered allocation of the lean kernel's probe scratch failed");
+        return launched(e, "trace kernel launch failed", launches);
     }
-    for (; n > 0; n--, p++) h = (h ^ *p) * 0x100000001B3ull;
-    return h;
-}
-
-// what a verdict depends on: the prescription, the media / index tables, and the description of the bundle where the
-// library has one (`bundle_key`: on-device sources; rays that arrive as arrays are the caller's business -- see above)
-unsigned long long verdict_key(const rtb::TraceParams &P, unsigned long long bundle_key)
-{
-    unsigned long long h = 0xcbf29ce484222325ull ^ bundle_key;
-    h = hash_bytes(h, &P.n_surf, sizeof(P.n_surf));
-    h = hash_bytes(h, &P.n_wl, sizeof(P.n_wl));
-    h = hash_bytes(h, P.surf, sizeof(rtb::DevSurface) * (size_t)P.n_surf);
-    h = hash_bytes(h, P.mat, sizeof(rtb::DevMaterial) * (size_t)(P.n_surf + 1));
-    if (P.n_wl > 0) {
-        h = hash_bytes(h, P.wl, sizeof(double) * (size_t)P.n_wl);
-        h = hash_bytes(h, P.n_tab, sizeof(double) * (size_t)(P.n_wl + 1) * (size_t)(P.n_surf + 1));
-    }
-    return h ? h : 1ull;
-}
-
-// (the whole description, first ray and count included: the rays of such a launch are a pure function of the key, so a
-// verdict, once read back, is final -- launch() then drops the probe)
-unsigned long long source_key(const rtb::DevSource *list, int n, long long n_rays)
-{
-    unsigned long long h = 0x84222325cbf29ce4ull;
-    h = hash_bytes(h, &n_rays, sizeof(n_rays));
-    for (int k = 0; k < n; k++) h = hash_bytes(h, &list[k], sizeof(list[k]));
-    return h ? h : 1ull;
-}
-
-// Consume a finished read-back, then say which kernel this launch should use.  Returns the entry that may take this
-// launch's read-back (NULL: none free, or caching is off).
-VerdictEntry *verdict_lookup(DeviceCtx *ctx, unsigned long long key, int n_src, int *pure_mode, unsigned long long *general)
-{
-    *pure_mode = 0;
-    *general = 0ull;
-    if (n_src > kVerdictMaxSources) return nullptr;
-    VerdictEntry *e = nullptr, *victim = nullptr;
-    for (VerdictEntry &v : ctx->verdict) {
-        if (v.used && v.key == key) {
-            e = &v;
-            break;
-        }
-        // (a slot whose read-back is still in flight keeps its buffer); else: an unused slot, or the least recently used
-        if (v.used && v.pending && cudaEventQuery(v.ev) != cudaSuccess) continue;
-        if (!victim || (victim->used && (!v.used || v.stamp < victim->stamp))) victim = &v;
-    }
-    cudaGetLastError();                   // (cudaErrorNotReady from the queries is not an error)
-    if (!e) {
-        if (!victim) return nullptr;
-        e = victim;
-        unsigned *pin = e->pin;
-        const int pin_sources = e->pin_sources;
-        cudaEvent_t ev = e->ev;
-        *e = VerdictEntry();
-        e->pin = pin;
-        e->pin_sources = pin_sources;
-        e->ev = ev;
-        e->used = true;
-        e->key = key;
-        if (e->pin_sources < n_src) {
-            if (e->pin) cudaFreeHost(e->pin);
-            e->pin = nullptr;
-            e->pin_sources = 0;
-            if (cudaHostAlloc((void **)&e->pin, sizeof(unsigned) * 2 * rtb::kMaxSurfaces * (size_t)n_src,
-                              cudaHostAllocDefault) != cudaSuccess) {
-                cudaGetLastError();
-                e->used = false;
-                return nullptr;
-            }
-            e->pin_sources = n_src;
-        }
-        if (!e->ev && cudaEventCreateWithFlags(&e->ev, cudaEventDisableTiming) != cudaSuccess) {
-            cudaGetLastError();
-            e->used = false;
-            return nullptr;
-        }
-    }
-    e->stamp = ++ctx->verdict_clock;
-    if (e->pending) {
-        const cudaError_t q = cudaEventQuery(e->ev);
-        if (q == cudaSuccess) {
-            const unsigned long long g = rtb::lean_verdict_from_counts(e->pin, e->pending_n_src, e->pending_n_surf);
-            if (e->have && g != e->general) {
-                e->flips++;
-                e->stable = 0;
-            } else if (++e->stable >= 16) {
-                e->flips = 0;
-            }
-            e->general = g;
-            e->have = true;
-            e->pending = false;
-        } else if (q != cudaErrorNotReady) {
-            e->pending = false;           // (the stream died: forget the read-back)
-        }
-        cudaGetLastError();
-    }
-    if (e->have && e->flips < 3) {
-        *pure_mode = 1;
-        *general = e->general;
-    }
-    return e->pending ? nullptr : e;
-}
-
-// `lean_counts`: probe scratch owned by the caller (the host pipeline's slots), or NULL to take it from the device's
-// stream-ordered pool for the duration of this launch.  `bundle_key`: see verdict_key.
-int launch(const rtb::TraceParams &P, int precision, DeviceCtx *ctx, int device, cudaStream_t stream,
-           unsigned *lean_counts = nullptr, unsigned long long bundle_key = 0ull)
-{
-    if (P.n_rays > 0 && wants_lean(P, precision)) {
-        const int n_src = std::max(P.n_src, 1);
-        const size_t bytes = sizeof(unsigned) * 2 * rtb::kMaxSurfaces * (size_t)n_src;
-        unsigned *counts = lean_counts;
-        if (!counts) {
-            int rc = ensure_pool(ctx, device);
-            if (rc) return rc;
-            if (cudaMallocFromPoolAsync((void **)&counts, bytes, ctx->pool, stream) != cudaSuccess)
-                return fail(RTB_ERR_NOMEM, "stream-ordered allocation of %zu bytes of probe scratch failed", bytes);
-        }
-        int launches = 0;
-        int pure_mode = (int)g_lean_pure.load(std::memory_order_relaxed);
-        unsigned long long general = 0ull;
-        VerdictEntry *entry = nullptr;
-        std::unique_lock<std::mutex> lock(ctx->verdict_mutex, std::defer_lock);
-        if (pure_mode == 1) {
-            // (a stream that is being captured into a graph can neither be queried nor read back from: no cache)
-            cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-            if (cudaStreamIsCapturing(stream, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone) {
-                cudaGetLastError();
-                pure_mode = 0;
-            } else {
-                lock.lock();
-                entry = verdict_lookup(ctx, verdict_key(P, bundle_key), n_src, &pure_mode, &general);
-            }
-        }
-        bool pure_used = false, probed = false;
-        // (on-device sources: the key determines the rays, the verdict that came back for it is final)
-        const bool final_verdict = bundle_key != 0ull && pure_mode == 1 &&
-                                   !g_keep_probe_counts.load(std::memory_order_relaxed);
-        cudaError_t e = rtb::launch_trace_lean(P, counts, ctx->sm_count, stream, &launches, pure_mode, general, &pure_used,
-                                               final_verdict, &probed);
-        static const bool debug = getenv("RTB_LEAN_DEBUG") != nullptr;
-        if (debug)
-            fprintf(stderr, "[rtb] lean launch: %lld rays x %d src, mode %d, verdict %#llx, entry %p -> %s\n", (long long)P.n_rays,
-                    n_src, pure_mode, general, (void *)entry, pure_used ? "pure" : "probe-driven");
-        if (e == cudaSuccess && entry && probed) {
-            // this launch's probe counts, for the next launch of the same key
-            if (cudaMemcpyAsync(entry->pin, counts, bytes, cudaMemcpyDeviceToHost, stream) == cudaSuccess &&
-                cudaEventRecord(entry->ev, stream) == cudaSuccess) {
-                entry->pending = true;
-                entry->pending_n_src = n_src;
-                entry->pending_n_surf = P.n_surf;
-            } else {
-                cudaGetLastError();
-            }
-        }
-        if (lock.owns_lock()) lock.unlock();
-        if (pure_used) g_pure_launches.fetch_add(1, std::memory_order_relaxed);
-        if (e == cudaSuccess && g_keep_probe_counts.load(std::memory_order_relaxed))
-            e = cudaMemcpyAsync(g_last_probe_counts, counts, sizeof(g_last_probe_counts), cudaMemcpyDeviceToHost, stream),
-            cudaStreamSynchronize(stream);
-        if (!lean_counts) cudaFreeAsync(counts, stream);
-        if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "trace kernel launch failed: %s", cudaGetErrorString(e));
-        g_launches.fetch_add(launches, std::memory_order_relaxed);
-        return RTB_OK;
-    }
-    cudaError_t e = (precision == RTB_F64_EXACT) ? rtb::launch_trace_f64(P, ctx->sm_count, stream)
-                                                 : rtb::launch_trace_fast(P, precision, ctx->sm_count, stream);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "trace kernel launch failed: %s", cudaGetErrorString(e));
-    if (P.n_rays > 0) g_launches.fetch_add(1, std::memory_order_relaxed);
-    return RTB_OK;
+    const cudaError_t e = (precision == RTB_F64_EXACT) ? rtb::launch_trace_f64(P, ctx->sm_count, stream)
+                                                       : rtb::launch_trace_fast(P, precision, ctx->sm_count, stream);
+    return launched(e, "trace kernel launch failed", P.n_rays > 0 ? 1 : 0);
 }
 
 int grow_dev(double **p, size_t *have, size_t want)
@@ -720,55 +539,15 @@ int rtb_device_count(void)
 
 int64_t rtb_launch_count(void) { return g_launches.load(); }
 
-int64_t rtb_pure_launch_count(void) { return g_pure_launches.load(); }
-
-int rtb_last_probe_counts(uint32_t *out, int n_surfaces)
-{
-    if (!out || n_surfaces < 0 || n_surfaces > RTB_MAX_SURFACES) return fail(RTB_ERR_INVALID, "bad arguments");
-    for (int k = 0; k < 2 * n_surfaces; k++) out[k] = g_last_probe_counts[k];
-    return RTB_OK;
-}
-
 int rtb_tune(const char *key, int64_t value)
 {
     if (!key) return fail(RTB_ERR_INVALID, "key is NULL");
-    if (strcmp(key, "lean_min_rays") == 0) {
-        g_lean_min_rays.store(value, std::memory_order_relaxed);
-        return RTB_OK;
-    }
-    if (strcmp(key, "psf_dmma") == 0) {
-        rtb::set_psf_dmma((int)value);
-        return RTB_OK;
-    }
-    if (strcmp(key, "lean_min_share_pct") == 0) {
-        rtb::set_lean_min_share_pct((int)value);
-        return RTB_OK;
-    }
-    if (strcmp(key, "lean_pure") == 0) {
-        if (value < 0 || value > 2) return fail(RTB_ERR_INVALID, "lean_pure takes 0, 1 or 2");
-        g_lean_pure.store(value, std::memory_order_relaxed);
+    for (const Knob &k : kKnobs) {
+        if (strcmp(key, k.key) != 0) continue;
+        if (value < k.lo || value > k.hi) return fail(RTB_ERR_INVALID, "%s takes %lld .. %lld", key, k.lo, k.hi);
+        k.value->store(value, std::memory_order_relaxed);
         // (setting the mode also forgets every cached verdict: tests start from a known state)
-        for (DeviceCtx &c : g_ctx) {
-            if (!c.ready) continue;
-            std::lock_guard<std::mutex> lock(c.verdict_mutex);
-            for (VerdictEntry &v : c.verdict) {
-                if (v.used && v.pending) cudaEventSynchronize(v.ev);
-                v.used = v.have = v.pending = false;
-            }
-            cudaGetLastError();
-        }
-        return RTB_OK;
-    }
-    if (strcmp(key, "sweep_split_rays") == 0) {
-        g_sweep_split_rays.store(value, std::memory_order_relaxed);
-        return RTB_OK;
-    }
-    if (strcmp(key, "keep_probe_counts") == 0) {
-        g_keep_probe_counts.store(value, std::memory_order_relaxed);
-        return RTB_OK;
-    }
-    if (strcmp(key, "host_fail_chunk") == 0) {
-        g_host_fail_chunk.store(value, std::memory_order_relaxed);
+        if (k.value == &rtb::g_lean_pure) rtb::lean_forget_verdicts();
         return RTB_OK;
     }
     return fail(RTB_ERR_INVALID, "unknown tuning key '%s'", key);
@@ -783,15 +562,13 @@ int rtb_trace_device(const rtb_system *sys, const double *rays_in_dev, int64_t n
     if (n_rays < 0) return fail(RTB_ERR_INVALID, "n_rays = %lld is negative", (long long)n_rays);
     if (n_rays > 0 && !rays_in_dev) return fail(RTB_ERR_INVALID, "rays_in_dev is NULL");
     if (n_rays > 0 && P.any_store && !out_dev) return fail(RTB_ERR_INVALID, "out_dev is NULL but the keep mode stores rays");
-    DeviceCtx *ctx;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
+    OnDevice on;
+    if ((rc = on.enter(device))) return rc;
     P.rays_in = rays_in_dev;
     P.out = out_dev;
     P.n_rays = n_rays;
     P.out_stride = 8 * (long long)n_rays;
-    return launch(P, opts->precision, ctx, device, (cudaStream_t)stream);
+    return launch(P, opts->precision, on, (cudaStream_t)stream);
 }
 
 int rtb_trace_source(const rtb_system *sys, const rtb_source *src, int64_t first_ray, int64_t n_rays,
@@ -802,15 +579,13 @@ int rtb_trace_source(const rtb_system *sys, const rtb_source *src, int64_t first
     if (rc) return rc;
     if ((rc = pack_source(src, first_ray, n_rays, P.src))) return rc;
     if (n_rays > 0 && P.any_store && !out_dev) return fail(RTB_ERR_INVALID, "out_dev is NULL but the keep mode stores rays");
-    DeviceCtx *ctx;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
+    OnDevice on;
+    if ((rc = on.enter(device))) return rc;
     P.rays_in = nullptr;
     P.out = out_dev;
     P.n_rays = n_rays;
     P.out_stride = 8 * (long long)n_rays;
-    return launch(P, opts->precision, ctx, device, (cudaStream_t)stream, nullptr, source_key(&P.src, 1, P.n_rays));
+    return launch(P, opts->precision, on, (cudaStream_t)stream, nullptr, &P.src);
 }
 
 int rtb_trace_sources(const rtb_system *sys, const rtb_source *srcs, int32_t n_src, int64_t first_ray,
@@ -829,40 +604,35 @@ int rtb_trace_sources(const rtb_system *sys, const rtb_source *srcs, int32_t n_s
         if ((rc = pack_source(srcs + k, first_ray, n_rays_each, list[(size_t)k]))) return rc;
     if (n_rays_each == 0) return RTB_OK;
     if (P.any_store && !out_dev) return fail(RTB_ERR_INVALID, "out_dev is NULL but the keep mode stores rays");
-    DeviceCtx *ctx;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
+    OnDevice on;
+    if ((rc = on.enter(device))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    {
-        wants_lean(P, opts->precision);          // (reads the environment once)
-        const long long split = g_sweep_split_rays.load(std::memory_order_relaxed);
-        if (n_src > 1 && split >= 0 && n_rays_each >= split) {
-            // one launch per source: rows [k n, (k + 1) n) of every kept slab, bucket k of the reductions
-            const bool planes_out = (opts->flags & RTB_FLAG_PLANES_OUT) != 0;
-            for (int k = 0; k < n_src; k++) {
-                rtb::TraceParams Q = P;
-                Q.src = list[(size_t)k];
-                Q.src_list = nullptr;
-                Q.n_src = 0;
-                Q.rays_in = nullptr;
-                Q.out = out_dev ? out_dev + (size_t)k * (size_t)n_rays_each * (planes_out ? 1 : 8) : nullptr;
-                Q.n_rays = n_rays_each;
-                Q.out_stride = 8 * (long long)n_rays_each * n_src;
-                if (Q.red.stats) Q.red.stats += (long long)k * RTB_N_STATS;
-                if (Q.red.grid) Q.red.grid += (long long)k * 3 * Q.red.grid_n * Q.red.grid_n;
-                rtb::finish_reduce(Q.red);
-                if ((rc = launch(Q, opts->precision, ctx, device, st, nullptr, source_key(&list[(size_t)k], 1, n_rays_each)))) return rc;
-            }
-            return RTB_OK;
+    const long long split = g_sweep_split_rays.load(std::memory_order_relaxed);
+    if (n_src > 1 && split >= 0 && n_rays_each >= split) {
+        // one launch per source: rows [k n, (k + 1) n) of every kept slab, bucket k of the reductions
+        const bool planes_out = (opts->flags & RTB_FLAG_PLANES_OUT) != 0;
+        for (int k = 0; k < n_src; k++) {
+            rtb::TraceParams Q = P;
+            Q.src = list[(size_t)k];
+            Q.src_list = nullptr;
+            Q.n_src = 0;
+            Q.rays_in = nullptr;
+            Q.out = out_dev ? out_dev + (size_t)k * (size_t)n_rays_each * (planes_out ? 1 : 8) : nullptr;
+            Q.n_rays = n_rays_each;
+            Q.out_stride = 8 * (long long)n_rays_each * n_src;
+            if (Q.red.stats) Q.red.stats += (long long)k * RTB_N_STATS;
+            if (Q.red.grid) Q.red.grid += (long long)k * 3 * Q.red.grid_n * Q.red.grid_n;
+            rtb::finish_reduce(Q.red);
+            if ((rc = launch(Q, opts->precision, on, st, nullptr, &list[(size_t)k]))) return rc;
         }
+        return RTB_OK;
     }
     // the list lives in stream-ordered device memory for exactly this launch (pageable source: the copy has staged
     // it by the time the call returns, so the vector may go out of scope)
     rtb::DevSource *list_dev = nullptr;
     const size_t bytes = sizeof(rtb::DevSource) * (size_t)n_src;
-    if ((rc = ensure_pool(ctx, device))) return rc;
-    if (cudaMallocFromPoolAsync((void **)&list_dev, bytes, ctx->pool, st) != cudaSuccess)
+    if ((rc = ensure_pool(on.ctx, device))) return rc;
+    if (cudaMallocFromPoolAsync((void **)&list_dev, bytes, on.ctx->pool, st) != cudaSuccess)
         return fail(RTB_ERR_NOMEM, "stream-ordered allocation of %zu bytes for the source list failed", bytes);
     cudaError_t e = cudaMemcpyAsync(list_dev, list.data(), bytes, cudaMemcpyHostToDevice, st);
     if (e != cudaSuccess) {
@@ -876,7 +646,7 @@ int rtb_trace_sources(const rtb_system *sys, const rtb_source *srcs, int32_t n_s
     P.out = out_dev;
     P.n_rays = n_rays_each;
     P.out_stride = 8 * (long long)n_rays_each * n_src;
-    rc = launch(P, opts->precision, ctx, device, st, nullptr, source_key(list.data(), n_src, n_rays_each));
+    rc = launch(P, opts->precision, on, st, nullptr, list.data());
     cudaFreeAsync(list_dev, st);
     return rc;
 }
@@ -894,10 +664,9 @@ int rtb_trace_host(const rtb_system *sys, const double *rays_in_host, int64_t n_
         return fail(RTB_ERR_UNSUPPORTED, "the plane (8, N) layouts are offered by the device entry points only");
     const int slabs = n_out_slabs(sys, opts);
     if (slabs > 0 && !out_host) return fail(RTB_ERR_INVALID, "out_host is NULL but the keep mode stores rays");
-    DeviceCtx *ctx;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
+    OnDevice on;
+    if ((rc = on.enter(device))) return rc;
+    DeviceCtx *ctx = on.ctx;
     std::lock_guard<std::mutex> lock(ctx->host_path);
 
     // chunk so that one chunk's output is ~64 MiB (RTB_HOST_CHUNK_MIB overrides; 8-128 MiB measured within 15%): big enough for PCIe efficiency,
@@ -922,7 +691,7 @@ int rtb_trace_host(const rtb_system *sys, const double *rays_in_host, int64_t n_
         if (!sl.stream) RTB_CUDA(cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
         if (!sl.done) RTB_CUDA(cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming));
         if (!sl.copied_in) RTB_CUDA(cudaEventCreateWithFlags(&sl.copied_in, cudaEventDisableTiming));
-        if (!sl.lean_counts) RTB_CUDA(cudaMalloc((void **)&sl.lean_counts, sizeof(unsigned) * 2 * rtb::kMaxSurfaces));
+        if (!sl.lean_scratch) RTB_CUDA(cudaMalloc(&sl.lean_scratch, rtb::lean_scratch_bytes(1)));
         if ((rc = grow_dev(&sl.dev_in, &sl.dev_in_bytes, (size_t)chunk * row))) return rc;
         if (slabs > 0 && (rc = grow_dev(&sl.dev_out, &sl.dev_out_bytes, (size_t)chunk * row * slabs))) return rc;
         if (!in_pinned && (rc = grow_pin(&sl.pin_in, &sl.pin_in_bytes, (size_t)chunk * row))) return rc;
@@ -1023,7 +792,7 @@ int rtb_trace_host(const rtb_system *sys, const double *rays_in_host, int64_t n_
             P.out_stride = 8 * cnt;
             if (c == g_host_fail_chunk.load(std::memory_order_relaxed))
                 return fail(RTB_ERR_CUDA, "injected failure before the launch of chunk %lld (rtb_tune host_fail_chunk)", c);
-            if ((rc = launch(P, opts->precision, ctx, device, sl.stream, sl.lean_counts))) return rc;
+            if ((rc = launch(P, opts->precision, on, sl.stream, sl.lean_scratch))) return rc;
             if (!lag) {
                 if ((rc = copy_out(c))) return rc;
             } else if (c > 0) {
@@ -1052,24 +821,18 @@ int rtb_generate_device(const rtb_source *src, int64_t first_ray, int64_t n_rays
     if (rc) return rc;
     if (n_rays == 0) return RTB_OK;
     if (!rays_out_dev) return fail(RTB_ERR_INVALID, "rays_out_dev is NULL");
-    DeviceCtx *ctx;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
-    cudaError_t e = rtb::launch_generate(d, n_rays, rays_out_dev, ctx->sm_count, (cudaStream_t)stream);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "generator launch failed: %s", cudaGetErrorString(e));
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return RTB_OK;
+    OnDevice on;
+    if ((rc = on.enter(device))) return rc;
+    return launched(rtb::launch_generate(d, n_rays, rays_out_dev, on.ctx->sm_count, (cudaStream_t)stream),
+                    "generator launch failed", 1);
 }
 
 int rtb_reduce_init(const rtb_reduce *red, int device, void *stream)
 {
     if (!red) return fail(RTB_ERR_INVALID, "reduce pointer is NULL");
-    DeviceCtx *ctx;
+    OnDevice on;
     int rc;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
+    if ((rc = on.enter(device))) return rc;
     rtb::DevReduce d;
     memset(&d, 0, sizeof(d));
     d.stats = red->stats_dev;
@@ -1077,10 +840,7 @@ int rtb_reduce_init(const rtb_reduce *red, int device, void *stream)
     d.grid_n = red->grid_n;
     rtb::finish_reduce(d);
     if (!d.stats && !d.grid) return RTB_OK;
-    cudaError_t e = rtb::launch_reduce_init(d, ctx->sm_count, (cudaStream_t)stream);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "reduce-init launch failed: %s", cudaGetErrorString(e));
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return RTB_OK;
+    return launched(rtb::launch_reduce_init(d, on.ctx->sm_count, (cudaStream_t)stream), "reduce-init launch failed", 1);
 }
 
 int rtb_intersect_rays_device(const double *ray1_dev, int64_t n1, const double *ray2_dev, int64_t n2,
@@ -1088,19 +848,13 @@ int rtb_intersect_rays_device(const double *ray1_dev, int64_t n1, const double *
 {
     if (n1 < 0 || n2 < 0) return fail(RTB_ERR_INVALID, "negative ray count");
     if (!(n1 == n2 || n1 == 1 || n2 == 1)) return fail(RTB_ERR_INVALID, "ray1 and ray2 must be the same length");
-    const long long n = std::max<long long>(n1, n2);
     if (n1 == 0 || n2 == 0) return RTB_OK;
     if (!ray1_dev || !ray2_dev || !pts_out_dev) return fail(RTB_ERR_INVALID, "NULL device pointer");
-    DeviceCtx *ctx;
+    OnDevice on;
     int rc;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
-    (void)n;
-    cudaError_t e = rtb::launch_intersect(ray1_dev, n1, ray2_dev, n2, pts_out_dev, (cudaStream_t)stream);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "intersect launch failed: %s", cudaGetErrorString(e));
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return RTB_OK;
+    if ((rc = on.enter(device))) return rc;
+    return launched(rtb::launch_intersect(ray1_dev, n1, ray2_dev, n2, pts_out_dev, (cudaStream_t)stream),
+                    "intersect launch failed", 1);
 }
 
 int rtb_ray2plane_device(const double *rays_dev, int64_t n_rays, const double *normal_dev, int64_t n_normal,
@@ -1113,16 +867,12 @@ int rtb_ray2plane_device(const double *rays_dev, int64_t n_rays, const double *n
         return fail(RTB_ERR_INVALID, "normal / center must have 1 or n_rays rows");
     if (!rays_dev || !normal_dev || !center_dev || !index_dev || !rays_out_dev || !ts_out_dev)
         return fail(RTB_ERR_INVALID, "NULL device pointer");
-    DeviceCtx *ctx;
+    OnDevice on;
     int rc;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
-    cudaError_t e = rtb::launch_ray2plane(rays_dev, n_rays, normal_dev, n_normal, center_dev, n_center, index_dev,
-                                          exclude_backward, rays_out_dev, ts_out_dev, (cudaStream_t)stream);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "ray2plane launch failed: %s", cudaGetErrorString(e));
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return RTB_OK;
+    if ((rc = on.enter(device))) return rc;
+    return launched(rtb::launch_ray2plane(rays_dev, n_rays, normal_dev, n_normal, center_dev, n_center, index_dev,
+                                          exclude_backward, rays_out_dev, ts_out_dev, (cudaStream_t)stream),
+                    "ray2plane launch failed", 1);
 }
 
 int rtb_distinct_wavelengths_device(const double *rays_dev, int64_t n_rays, double *table_dev,
@@ -1131,17 +881,15 @@ int rtb_distinct_wavelengths_device(const double *rays_dev, int64_t n_rays, doub
     if (n_rays < 0) return fail(RTB_ERR_INVALID, "n_rays is negative");
     if (!table_dev || !wavelengths_host || !n_found) return fail(RTB_ERR_INVALID, "NULL pointer");
     if (n_rays > 0 && !rays_dev) return fail(RTB_ERR_INVALID, "rays_dev is NULL");
-    DeviceCtx *ctx;
+    OnDevice on;
     int rc;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
+    if ((rc = on.enter(device))) return rc;
     int found = 0;
     double vals[RTB_MAX_WAVELENGTHS + 1];
-    cudaError_t e = rtb::run_distinct_wavelengths(rays_dev, n_rays, table_dev, RTB_MAX_WAVELENGTHS + 1, vals, &found,
-                                                  ctx->sm_count, (cudaStream_t)stream);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "distinct-wavelength scan failed: %s", cudaGetErrorString(e));
-    g_launches.fetch_add(n_rays > 0 ? 2 : 1, std::memory_order_relaxed);
+    if ((rc = launched(rtb::run_distinct_wavelengths(rays_dev, n_rays, table_dev, RTB_MAX_WAVELENGTHS + 1, vals, &found,
+                                                     on.ctx->sm_count, (cudaStream_t)stream),
+                       "distinct-wavelength scan failed", n_rays > 0 ? 2 : 1)))
+        return rc;
     std::sort(vals, vals + found);
     for (int k = 0; k < found; k++) wavelengths_host[k] = vals[k];
     *n_found = found;
@@ -1213,32 +961,26 @@ int rtb_psf_from_grid_device(const double *grid_dev, int grid_n, double grid_hal
     if (!psf_out_dev && !(field_re_dev && field_im_dev)) return fail(RTB_ERR_INVALID, "psf: no output requested");
     if (!scratch_dev || scratch_doubles < rtb::psf_scratch_doubles(grid_n, n_samples, normalize_by_count))
         return fail(RTB_ERR_INVALID, "psf: scratch buffer too small (see rtb_psf_scratch_doubles)");
-    DeviceCtx *ctx;
+    OnDevice on;
     int rc;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
+    if ((rc = on.enter(device))) return rc;
     int launches = 0;
     cudaError_t e = rtb::launch_psf(grid_dev, grid_n, grid_half_width, n_samples, df, normalize_by_count, scratch_dev,
-                                    psf_out_dev, field_re_dev, field_im_dev, ctx->sm_count, (cudaStream_t)stream,
+                                    psf_out_dev, field_re_dev, field_im_dev, on.ctx->sm_count, (cudaStream_t)stream,
                                     &launches);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "psf launch failed: %s", cudaGetErrorString(e));
-    g_launches.fetch_add(launches, std::memory_order_relaxed);
-    return RTB_OK;
+    return launched(e, "psf launch failed", launches);
 }
 
 int rtb_selftest_exact_math(int device, uint64_t seed, int64_t n_cases, uint64_t mismatches[3])
 {
     if (!mismatches || n_cases < 0) return fail(RTB_ERR_INVALID, "bad arguments");
-    DeviceCtx *ctx;
+    OnDevice on;
     int rc;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
+    if ((rc = on.enter(device))) return rc;
     unsigned long long bad[3] = {0, 0, 0};
-    cudaError_t e = rtb::run_exact_math_selftest(seed, n_cases, bad, ctx->sm_count);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "exact-math self-test failed to run: %s", cudaGetErrorString(e));
-    g_launches.fetch_add(1, std::memory_order_relaxed);
+    if ((rc = launched(rtb::run_exact_math_selftest(seed, n_cases, bad, on.ctx->sm_count),
+                       "exact-math self-test failed to run", 1)))
+        return rc;
     for (int k = 0; k < 3; k++) mismatches[k] = bad[k];
     return RTB_OK;
 }
@@ -1246,14 +988,11 @@ int rtb_selftest_exact_math(int device, uint64_t seed, int64_t n_cases, uint64_t
 int rtb_measure_dfma_rate(int device, double *dfma_per_s, double *elapsed_ms)
 {
     if (!dfma_per_s) return fail(RTB_ERR_INVALID, "dfma_per_s is NULL");
-    DeviceCtx *ctx;
+    OnDevice on;
     int rc;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
+    if ((rc = on.enter(device))) return rc;
     double ms = 0;
-    cudaError_t e = rtb::run_dfma_probe(ctx->sm_count, dfma_per_s, &ms);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "DFMA probe failed: %s", cudaGetErrorString(e));
+    if ((rc = launched(rtb::run_dfma_probe(on.ctx->sm_count, dfma_per_s, &ms), "DFMA probe failed", 0))) return rc;
     if (elapsed_ms) *elapsed_ms = ms;
     return RTB_OK;
 }
@@ -1262,14 +1001,12 @@ int rtb_measure_dfma_chain_rate(int device, int chains, double *dfma_per_s, doub
 {
     if (!dfma_per_s) return fail(RTB_ERR_INVALID, "dfma_per_s is NULL");
     if (chains != 1 && chains != 2 && chains != 4 && chains != 8) return fail(RTB_ERR_INVALID, "chains must be 1, 2, 4 or 8");
-    DeviceCtx *ctx;
+    OnDevice on;
     int rc;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
+    if ((rc = on.enter(device))) return rc;
     double ms = 0;
-    cudaError_t e = rtb::run_dfma_chain_probe(ctx->sm_count, chains, dfma_per_s, &ms);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "DFMA chain probe failed: %s", cudaGetErrorString(e));
+    if ((rc = launched(rtb::run_dfma_chain_probe(on.ctx->sm_count, chains, dfma_per_s, &ms), "DFMA chain probe failed", 0)))
+        return rc;
     if (elapsed_ms) *elapsed_ms = ms;
     return RTB_OK;
 }
@@ -1277,14 +1014,10 @@ int rtb_measure_dfma_chain_rate(int device, int chains, double *dfma_per_s, doub
 int rtb_measure_copy_bandwidth(int device, int64_t bytes, double *bytes_per_s)
 {
     if (!bytes_per_s || bytes <= 0) return fail(RTB_ERR_INVALID, "bad arguments");
-    DeviceCtx *ctx;
+    OnDevice on;
     int rc;
-    if ((rc = get_ctx(device, &ctx))) return rc;
-    DeviceGuard guard;
-    if ((rc = guard.enter(device))) return rc;
-    cudaError_t e = rtb::run_copy_probe(bytes, bytes_per_s);
-    if (e != cudaSuccess) return fail(RTB_ERR_CUDA, "copy probe failed: %s", cudaGetErrorString(e));
-    return RTB_OK;
+    if ((rc = on.enter(device))) return rc;
+    return launched(rtb::run_copy_probe(bytes, bytes_per_s), "copy probe failed", 0);
 }
 
 void *rtb_host_alloc(size_t bytes)

@@ -21,6 +21,10 @@ constexpr int kMaxSurfaces = RTB_MAX_SURFACES;
 constexpr int kMaxMedia = RTB_MAX_SURFACES + 1;
 constexpr int kMaxWavelengths = RTB_MAX_WAVELENGTHS;
 constexpr int kMaxSlabs = 2 * RTB_MAX_SURFACES + 1;
+constexpr int kMaxDevices = 64;       // device indices the C ABI accepts
+
+// sets rtb_last_error() and returns `code` (rtb_api.cu; every translation unit of the C ABI reports errors through it)
+int api_fail(int code, const char *fmt, ...);
 
 // launch shape of the trace kernels: 128-thread blocks, register budget for kTraceMinBlocks resident blocks per SM
 #ifndef RTB_TRACE_THREADS

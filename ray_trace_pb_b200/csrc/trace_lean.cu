@@ -16,8 +16,16 @@
 //     caller's stream.  Hints (rtb_surface.hints) are therefore not needed by this kernel.
 //   * Spot statistics are tallied per thread in shared memory (touched once per ray) instead of in 24 registers.
 //
+// Below the kernels, the host side of the launch policy: which launches this kernel takes (lean_takes), the verdict
+// cache that picks the pure or the probe-driven instantiation, and the launch (launch_lean) -- rtb_api.cu calls these.
+//
 // THIS TRANSLATION UNIT MUST BE COMPILED WITH -fmad=false (see trace_f64.cu).
+#include <atomic>
 #include <cmath>
+#include <cstdio>
+#include <cstdlib>
+#include <cstring>
+#include <mutex>
 #include <math_constants.h>
 
 #include "exact_math.cuh"
@@ -39,7 +47,14 @@ namespace {
 constexpr int kLeanThreads = RTB_LEAN_THREADS;
 constexpr int kLeanMinBlocks = RTB_LEAN_MIN_BLOCKS;
 constexpr int kProbeRays = 2048;          // sample size of the probe launch, per source
-constexpr unsigned kProbeOneIn = 200;     // a surface runs the general steps when more than 1 in 200 probe rays failed
+
+// the probe's rule, for the kernel and for the host's verdict: a surface runs the general steps when more than 1 in 200
+// of the probe rays that reached it failed their lean step there (`cnt`: the probe's {reached, failed} for the surface)
+__host__ __device__ inline bool probe_says_general(const unsigned *cnt)
+{
+    constexpr unsigned kProbeOneIn = 200;
+    return (unsigned long long)cnt[1] * kProbeOneIn > (unsigned long long)cnt[0];
+}
 
 // which step a surface runs (decided once per block: kind, axes, the reciprocal radius, the probe's counts)
 enum StepCode : int { kLeanSphere = 0, kLeanFlat = 1, kGeneralRefracting = 2, kGeneralMirror = 3, kGeneralLens = 4,
@@ -247,7 +262,7 @@ __device__ __forceinline__ bool surface_step(const DevSurface &s, SurfaceShared 
 //            achromat systems) -- it does not carry the perfect-lens, tilted-flat and mirror steps, whose mere presence
 //            costs the sphere loop 2 % through register allocation; 1: every step.  2 / 3: the PURE forms of 0 / of
 //            "every lean step": no general steps, no probe counts -- the launcher has made sure (from an earlier probe's
-//            verdict on the same system, rtb_api.cu) that every surface can run its lean step.  Nothing in them branches on
+//            verdict on the same system, cached below) that every surface can run its lean step.  Nothing in them branches on
 //            a value loaded from memory, which lets ptxas keep the loop indices in uniform registers and read the
 //            prescription through the uniform datapath (operands that cost no operand-port cycle, DESIGN.md 4a).
 template <bool USE_TABLE, bool FROM_SOURCE, bool SWEEP, bool PROBE, int KINDS>
@@ -287,10 +302,8 @@ __global__ void __launch_bounds__(kLeanThreads, kLeanMinBlocks) trace_lean_kerne
         // it for the careful path)
         bool general = ((P.lean_general >> k) & 1ull) != 0 ||
                        (!sane && (s.kind == RTB_SURF_SPHERE || s.kind == RTB_SURF_PERFECT_LENS));
-        if (!PROBE && KINDS < 2 && P.lean_counts) {
-            const unsigned *cnt = P.lean_counts + ((size_t)(SWEEP ? blockIdx.y : 0) * kMaxSurfaces + k) * 2;
-            general |= (unsigned long long)cnt[1] * kProbeOneIn > (unsigned long long)cnt[0];
-        }
+        if (!PROBE && KINDS < 2 && P.lean_counts)
+            general |= probe_says_general(P.lean_counts + ((size_t)(SWEEP ? blockIdx.y : 0) * kMaxSurfaces + k) * 2);
         s_c.surf[k].code = step_code(s, general);
     }
     __syncthreads();
@@ -559,11 +572,28 @@ cudaError_t launch_lean_pick(const TraceParams &P, unsigned blocks, unsigned *pr
 
 } // namespace
 
-// share of surfaces with a lean step below which a system stays with trace_f64.cu (rtb_tune "lean_min_share_pct")
-int g_lean_min_share_pct = 75;
-void set_lean_min_share_pct(int pct) { g_lean_min_share_pct = pct; }
+// ---- launch policy: which launches this kernel takes, and which of its instantiations traces them -------------------
+// The knobs (rtb_tune keys of the same names, include/rtb.h; rtb_api.cu sets them):
+// launches of at least this many rays go to this kernel; smaller ones are not worth a probe.  Negative = never.
+std::atomic<long long> g_lean_min_rays{32768};
+// share of surfaces with a lean step (per cent) below which a system stays with trace_f64.cu
+std::atomic<long long> g_lean_min_share_pct{75};
+// 0 = the probe-driven kernels only; 1 (default) = the pure kernels once an earlier probe of the same system and bundle
+// has said that every surface can run its lean step (the verdict cache below); 2 = the pure kernels whenever the
+// system has a lean step for every surface, whatever the bundle (tests)
+std::atomic<long long> g_lean_pure{1};
+// test hook: every lean launch synchronises and keeps its probe's counts (first source only) for rtb_last_probe_counts()
+std::atomic<long long> g_keep_probe_counts{0};
 
-// What the lean kernel traces: fp64 exact, nothing stored but the final slab (or nothing at all), no reduction or one at
+// probe scratch of a launch of `n_sources` sources: n_sources x kMaxSurfaces x {reached, failed}
+size_t lean_scratch_bytes(int n_sources) { return sizeof(unsigned) * 2 * kMaxSurfaces * (size_t)n_sources; }
+
+namespace {
+
+std::atomic<long long> g_pure_launches{0};
+unsigned g_last_probe_counts[2 * kMaxSurfaces];
+
+// What this kernel traces: fp64 exact, nothing stored but the final slab (or nothing at all), no reduction or one at
 // an after-surface slab, not the intersect-only operator.
 bool lean_eligible(const TraceParams &P)
 {
@@ -580,25 +610,11 @@ bool lean_eligible(const TraceParams &P)
         const DevSurface &s = P.surf[k];
         n_lean += has_lean_step(s);
     }
-    if (100 * n_lean < g_lean_min_share_pct * P.n_surf) return false;
+    if (100 * n_lean < g_lean_min_share_pct.load(std::memory_order_relaxed) * P.n_surf) return false;
     if (P.red.slab < 0 && !P.any_store) return false;      // nothing to do: leave it to the general kernel's conventions
     return P.n_surf > 0;
 }
 
-// The probe's rule, for the host: bit k is set when more than 1 in kProbeOneIn of the probe rays that reached surface k
-// failed their lean step there, in any source (`counts`: n_src x kMaxSurfaces x {reached, failed}, the probe's output).
-unsigned long long lean_verdict_from_counts(const unsigned *counts, int n_src, int n_surf)
-{
-    unsigned long long general = 0ull;
-    for (int j = 0; j < n_src; j++)
-        for (int k = 0; k < n_surf; k++) {
-            const unsigned *cnt = counts + ((size_t)j * kMaxSurfaces + k) * 2;
-            if ((unsigned long long)cnt[1] * kProbeOneIn > (unsigned long long)cnt[0]) general |= 1ull << k;
-        }
-    return general;
-}
-
-namespace {
 bool sane_reciprocal(const DevSurface &s)
 {
     const double den = (s.kind == RTB_SURF_PERFECT_LENS) ? s.focal_len : s.radius;
@@ -630,46 +646,16 @@ bool build_runs(TraceParams &P, unsigned long long general)
     }
     return all_lean;
 }
-} // namespace
 
-// `counts`: device scratch of n_sources * kMaxSurfaces * 2 unsigned for the probe (zeroed here), owned by the caller for
-// the duration of both launches.  *launches is increased by the number of kernels launched.
-// `pure_mode` 0: the probe-driven kernels.  1: the pure kernels, if the system allows, with `verdict_general` = the
-// surfaces at which an EARLIER probe of the same system and bundle found bundle-wide failures of the plain lean step
-// (rtb_api.cu's cache; on-axis flats among them run the zero-tolerant lean flat, anything else sends the launch back to the
-// probe-driven kernels).  2: the pure kernels with no verdict (tests: whatever fails is re-traced by redo_ray).  The probe
-// runs in every mode but one (see probe_optional) -- in the pure modes its counts only feed the caller's next verdict.
-// *pure_used says what ran.
-// `probe_optional`: the verdict is final for this launch (rays that are a pure function of the cache key): when the pure
-// kernels take it, the probe -- which would only confirm it -- is not launched.  *probed says whether it was.
-cudaError_t launch_trace_lean(const TraceParams &P_in, unsigned *counts, int sm_count, cudaStream_t stream, int *launches,
-                              int pure_mode, unsigned long long verdict_general, bool *pure_used, bool probe_optional,
-                              bool *probed)
+// The probe over a sample of the rays when `counts` is given (zeroed here; the trace reads them), then the trace.
+// *launches is increased by the number of kernels launched.
+cudaError_t probe_and_trace(TraceParams P, unsigned *counts, int sm_count, cudaStream_t stream, int *launches)
 {
-    if (pure_used) *pure_used = false;
-    if (probed) *probed = false;
-    if (P_in.n_rays <= 0) return cudaSuccess;
-    TraceParams P = P_in;
     const bool sweep = P.n_src > 0;
-    const int n_sources = sweep ? P.n_src : 1;
-    // surfaces without a lean step (tilted / decentred axes, mirrors, lenses) run the general steps
-    P.lean_general = 0ull;
-    for (int k = 0; k < P.n_surf; k++) {
-        const DevSurface &s = P.surf[k];
-        if (!has_lean_step(s)) P.lean_general |= 1ull << k;
-    }
-    P.lean_pure = 0;
-    if (pure_mode != 0 && P.lean_general == 0ull && build_runs(P, pure_mode == 1 ? verdict_general : 0ull))
-        P.lean_pure = 1;
-    else
-        build_runs(P, P.lean_general);
-    if (pure_used) *pure_used = P.lean_pure != 0;
-    if (P.lean_pure != 0 && probe_optional) counts = nullptr;
-    if (probed) *probed = counts != nullptr;
     cudaError_t e;
     P.lean_counts = nullptr;
     if (counts) {
-        e = cudaMemsetAsync(counts, 0, sizeof(unsigned) * 2 * kMaxSurfaces * (size_t)n_sources, stream);
+        e = cudaMemsetAsync(counts, 0, lean_scratch_bytes(sweep ? P.n_src : 1), stream);
         if (e != cudaSuccess) return e;
         TraceParams Q = P;
         const long long n_probe = P.n_rays < kProbeRays ? P.n_rays : kProbeRays;
@@ -681,7 +667,7 @@ cudaError_t launch_trace_lean(const TraceParams &P_in, unsigned *counts, int sm_
         const unsigned pb = (unsigned)((n_probe + kLeanThreads - 1) / kLeanThreads);
         e = launch_lean_pick<true>(Q, pb, counts, stream);
         if (e != cudaSuccess) return e;
-        if (launches) ++*launches;
+        ++*launches;
         P.lean_counts = counts;
     }
     long long blocks = (P.n_rays + kLeanThreads - 1) / kLeanThreads;
@@ -689,8 +675,270 @@ cudaError_t launch_trace_lean(const TraceParams &P_in, unsigned *counts, int sm_
     if (sweep) max_blocks = (max_blocks + P.n_src - 1) / P.n_src;
     if (blocks > max_blocks) blocks = max_blocks;
     e = launch_lean_pick<false>(P, (unsigned)blocks, nullptr, stream);
-    if (e == cudaSuccess && launches) ++*launches;
+    if (e == cudaSuccess) ++*launches;
+    return e;
+}
+
+// ---- the verdict cache (DESIGN.md 4a) ----------------------------------------------------------------------------
+// The pure instantiations branch on kernel parameters only, so the choice "can every surface of this system run its
+// lean step with this bundle" has to be made on the host before the launch -- but the probe's counts are on the device.
+// Every lean launch therefore copies its probe's counts to a pinned slot asynchronously (no synchronisation), and the
+// NEXT launch of the same system + bundle description picks its kernel by them.  A wrong verdict costs time, never a bit
+// of the result: rays that fail a lean step are re-traced by redo_ray in every kernel.  A key whose verdict keeps
+// changing (one system traced alternately with bundles of different character from device arrays) stays with the
+// probe-driven kernels.
+constexpr int kVerdictEntries = 128;
+constexpr int kVerdictMaxSources = 64;
+
+struct VerdictEntry {
+    unsigned long long key = 0;
+    bool used = false, have = false, pending = false;
+    unsigned long long general = 0;   // the last consumed probe's verdict (verdict_from_counts)
+    int flips = 0, stable = 0;
+    int pending_n_src = 0, pending_n_surf = 0;
+    unsigned *pin = nullptr;          // pin_sources x kMaxSurfaces x 2 counts, page-locked
+    int pin_sources = 0;
+    cudaEvent_t ev = nullptr;
+    unsigned long long stamp = 0;
+};
+
+struct VerdictCache {
+    std::mutex mutex;
+    VerdictEntry entry[kVerdictEntries];
+    unsigned long long clock = 0;
+};
+
+VerdictCache g_verdicts[kMaxDevices];
+
+// 64-bit mix of a byte range (8 bytes at a time; the tail byte-wise)
+unsigned long long hash_bytes(unsigned long long h, const void *data, size_t n)
+{
+    const unsigned char *p = (const unsigned char *)data;
+    for (; n >= 8; n -= 8, p += 8) {
+        unsigned long long w;
+        memcpy(&w, p, 8);
+        h = (h ^ w) * 0x9E3779B97F4A7C15ull;
+        h ^= h >> 29;
+    }
+    for (; n > 0; n--, p++) h = (h ^ *p) * 0x100000001B3ull;
+    return h;
+}
+
+// what a verdict depends on: the prescription, the media / index tables, and the description of the bundle where the
+// library has one (`bundle_key`: on-device sources; rays that arrive as arrays are the caller's business -- see above)
+unsigned long long verdict_key(const TraceParams &P, unsigned long long bundle_key)
+{
+    unsigned long long h = 0xcbf29ce484222325ull ^ bundle_key;
+    h = hash_bytes(h, &P.n_surf, sizeof(P.n_surf));
+    h = hash_bytes(h, &P.n_wl, sizeof(P.n_wl));
+    h = hash_bytes(h, P.surf, sizeof(DevSurface) * (size_t)P.n_surf);
+    h = hash_bytes(h, P.mat, sizeof(DevMaterial) * (size_t)(P.n_surf + 1));
+    if (P.n_wl > 0) {
+        h = hash_bytes(h, P.wl, sizeof(double) * (size_t)P.n_wl);
+        h = hash_bytes(h, P.n_tab, sizeof(double) * (size_t)(P.n_wl + 1) * (size_t)(P.n_surf + 1));
+    }
+    return h ? h : 1ull;
+}
+
+// (the whole description, first ray and count included: the rays of such a launch are a pure function of the key, so a
+// verdict, once read back, is final -- launch_lean then drops the probe)
+unsigned long long source_key(const DevSource *list, int n, long long n_rays)
+{
+    unsigned long long h = 0x84222325cbf29ce4ull;
+    h = hash_bytes(h, &n_rays, sizeof(n_rays));
+    for (int k = 0; k < n; k++) h = hash_bytes(h, &list[k], sizeof(list[k]));
+    return h ? h : 1ull;
+}
+
+// bit k: the probe's rule says "general steps" at surface k, in any source (`counts`: the probe's output)
+unsigned long long verdict_from_counts(const unsigned *counts, int n_src, int n_surf)
+{
+    unsigned long long general = 0ull;
+    for (int j = 0; j < n_src; j++)
+        for (int k = 0; k < n_surf; k++)
+            if (probe_says_general(counts + ((size_t)j * kMaxSurfaces + k) * 2)) general |= 1ull << k;
+    return general;
+}
+
+// Consume a finished read-back, then say which kernel this launch should use.  Returns the entry that may take this
+// launch's read-back (NULL: none free, or caching is off).
+VerdictEntry *verdict_lookup(VerdictCache &cache, unsigned long long key, int n_src, int *pure_mode,
+                             unsigned long long *general)
+{
+    *pure_mode = 0;
+    *general = 0ull;
+    if (n_src > kVerdictMaxSources) return nullptr;
+    VerdictEntry *e = nullptr, *victim = nullptr;
+    for (VerdictEntry &v : cache.entry) {
+        if (v.used && v.key == key) {
+            e = &v;
+            break;
+        }
+        // (a slot whose read-back is still in flight keeps its buffer); else: an unused slot, or the least recently used
+        if (v.used && v.pending && cudaEventQuery(v.ev) != cudaSuccess) continue;
+        if (!victim || (victim->used && (!v.used || v.stamp < victim->stamp))) victim = &v;
+    }
+    cudaGetLastError();                   // (cudaErrorNotReady from the queries is not an error)
+    if (!e) {
+        if (!victim) return nullptr;
+        e = victim;
+        unsigned *pin = e->pin;
+        const int pin_sources = e->pin_sources;
+        cudaEvent_t ev = e->ev;
+        *e = VerdictEntry();
+        e->pin = pin;
+        e->pin_sources = pin_sources;
+        e->ev = ev;
+        e->used = true;
+        e->key = key;
+        if (e->pin_sources < n_src) {
+            if (e->pin) cudaFreeHost(e->pin);
+            e->pin = nullptr;
+            e->pin_sources = 0;
+            if (cudaHostAlloc((void **)&e->pin, lean_scratch_bytes(n_src), cudaHostAllocDefault) != cudaSuccess) {
+                cudaGetLastError();
+                e->used = false;
+                return nullptr;
+            }
+            e->pin_sources = n_src;
+        }
+        if (!e->ev && cudaEventCreateWithFlags(&e->ev, cudaEventDisableTiming) != cudaSuccess) {
+            cudaGetLastError();
+            e->used = false;
+            return nullptr;
+        }
+    }
+    e->stamp = ++cache.clock;
+    if (e->pending) {
+        const cudaError_t q = cudaEventQuery(e->ev);
+        if (q == cudaSuccess) {
+            const unsigned long long g = verdict_from_counts(e->pin, e->pending_n_src, e->pending_n_surf);
+            if (e->have && g != e->general) {
+                e->flips++;
+                e->stable = 0;
+            } else if (++e->stable >= 16) {
+                e->flips = 0;
+            }
+            e->general = g;
+            e->have = true;
+            e->pending = false;
+        } else if (q != cudaErrorNotReady) {
+            e->pending = false;           // (the stream died: forget the read-back)
+        }
+        cudaGetLastError();
+    }
+    if (e->have && e->flips < 3) {
+        *pure_mode = 1;
+        *general = e->general;
+    }
+    return e->pending ? nullptr : e;
+}
+
+} // namespace
+
+// whether this kernel takes the launch (else trace_f64.cu, or trace_fast.cu for the other precisions)
+bool lean_takes(const TraceParams &P, int precision)
+{
+    const long long min_rays = g_lean_min_rays.load(std::memory_order_relaxed);
+    return precision == RTB_F64_EXACT && P.n_rays > 0 && min_rays >= 0 && P.n_rays >= min_rays && lean_eligible(P);
+}
+
+// every device's cached verdicts (read-backs still in flight are waited for)
+void lean_forget_verdicts()
+{
+    for (VerdictCache &c : g_verdicts) {
+        std::lock_guard<std::mutex> lock(c.mutex);
+        for (VerdictEntry &v : c.entry) {
+            if (v.used && v.pending) {
+                cudaEventSynchronize(v.ev);
+                cudaGetLastError();
+            }
+            v.used = v.have = v.pending = false;
+        }
+    }
+}
+
+// A launch that lean_takes: the probe (unless the verdict makes it redundant) and the trace, on `stream`.
+// `scratch`: probe scratch of lean_scratch_bytes(1) owned by the caller (the host pipeline's slots), or NULL to take it
+// from `pool` for the duration of this launch -- cudaErrorMemoryAllocation if that fails.  `sources`: the host copy of
+// the source description(s) when the rays come from on-device sources (P.n_src of them for a sweep, else one): they
+// join the verdict's key.  NULL for rays from arrays.  *launches is increased by the number of kernels launched.
+cudaError_t launch_lean(const TraceParams &P_in, int device, int sm_count, cudaStream_t stream, cudaMemPool_t pool,
+                        void *scratch, const DevSource *sources, int *launches)
+{
+    TraceParams P = P_in;
+    const int n_src = P.n_src > 0 ? P.n_src : 1;
+    const size_t bytes = lean_scratch_bytes(n_src);
+    unsigned *counts = (unsigned *)scratch;
+    if (!counts && cudaMallocFromPoolAsync((void **)&counts, bytes, pool, stream) != cudaSuccess)
+        return cudaErrorMemoryAllocation;
+    const unsigned long long bundle_key = sources ? source_key(sources, n_src, P.n_rays) : 0ull;
+    int pure_mode = (int)g_lean_pure.load(std::memory_order_relaxed);
+    unsigned long long verdict = 0ull;
+    VerdictEntry *entry = nullptr;
+    VerdictCache &cache = g_verdicts[device];
+    std::unique_lock<std::mutex> lock(cache.mutex, std::defer_lock);
+    if (pure_mode == 1) {
+        // (a stream that is being captured into a graph can neither be queried nor read back from: no cache)
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        if (cudaStreamIsCapturing(stream, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone) {
+            cudaGetLastError();
+            pure_mode = 0;
+        } else {
+            lock.lock();
+            entry = verdict_lookup(cache, verdict_key(P, bundle_key), n_src, &pure_mode, &verdict);
+        }
+    }
+    // pure_mode 0: the probe-driven kernels.  1: the pure kernels, if the system allows, with `verdict` = the surfaces at
+    // which an EARLIER probe of the same system and bundle found bundle-wide failures of the plain lean step (on-axis
+    // flats among them run the zero-tolerant lean flat, anything else sends the launch back to the probe-driven
+    // kernels).  2: the pure kernels with no verdict (tests: whatever fails is re-traced by redo_ray).
+    // Surfaces without a lean step (tilted / decentred axes, mirrors, lenses) run the general steps.
+    P.lean_general = 0ull;
+    for (int k = 0; k < P.n_surf; k++)
+        if (!has_lean_step(P.surf[k])) P.lean_general |= 1ull << k;
+    P.lean_pure = pure_mode != 0 && P.lean_general == 0ull && build_runs(P, pure_mode == 1 ? verdict : 0ull);
+    if (!P.lean_pure) build_runs(P, P.lean_general);
+    // The probe runs in every mode -- in the pure kernels its counts only feed the next verdict -- but one: the rays of
+    // on-device sources are a pure function of the key, so a cached verdict the pure kernels take is final for them.
+    const bool keep_counts = g_keep_probe_counts.load(std::memory_order_relaxed) != 0;
+    const bool probed = !(P.lean_pure && sources && pure_mode == 1 && !keep_counts);
+    cudaError_t e = probe_and_trace(P, probed ? counts : nullptr, sm_count, stream, launches);
+    static const bool debug = getenv("RTB_LEAN_DEBUG") != nullptr;
+    if (debug)
+        fprintf(stderr, "[rtb] lean launch: %lld rays x %d src, mode %d, verdict %#llx, entry %p -> %s\n", (long long)P.n_rays,
+                n_src, pure_mode, verdict, (void *)entry, P.lean_pure ? "pure" : "probe-driven");
+    if (e == cudaSuccess && entry && probed) {
+        // this launch's probe counts, for the next launch of the same key
+        if (cudaMemcpyAsync(entry->pin, counts, bytes, cudaMemcpyDeviceToHost, stream) == cudaSuccess &&
+            cudaEventRecord(entry->ev, stream) == cudaSuccess) {
+            entry->pending = true;
+            entry->pending_n_src = n_src;
+            entry->pending_n_surf = P.n_surf;
+        } else {
+            cudaGetLastError();
+        }
+    }
+    if (lock.owns_lock()) lock.unlock();
+    if (P.lean_pure) g_pure_launches.fetch_add(1, std::memory_order_relaxed);
+    if (e == cudaSuccess && keep_counts)
+        e = cudaMemcpyAsync(g_last_probe_counts, counts, sizeof(g_last_probe_counts), cudaMemcpyDeviceToHost, stream),
+        cudaStreamSynchronize(stream);
+    if (!scratch) cudaFreeAsync(counts, stream);
     return e;
 }
 
 } // namespace rtb
+
+extern "C" {
+
+int64_t rtb_pure_launch_count(void) { return rtb::g_pure_launches.load(); }
+
+int rtb_last_probe_counts(uint32_t *out, int n_surfaces)
+{
+    if (!out || n_surfaces < 0 || n_surfaces > RTB_MAX_SURFACES) return rtb::api_fail(RTB_ERR_INVALID, "bad arguments");
+    for (int k = 0; k < 2 * n_surfaces; k++) out[k] = rtb::g_last_probe_counts[k];
+    return RTB_OK;
+}
+
+} // extern "C"
