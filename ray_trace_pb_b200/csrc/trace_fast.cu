@@ -17,7 +17,8 @@
 // below) but NOT in the validity masks of knife-edge rays: the reference's absolute 1e-12 on-surface test culls a few
 // rays in 1e5 purely on round-off (SURVEY.md section 0), which only the exact mode reproduces.
 //
-// Stated tolerances against the exact mode (asserted in tests/test_gpu_parity.py::test_fast_modes_tolerance):
+// Stated tolerances against the exact mode (asserted in tests/test_gpu_parity.py::test_fast_modes_tolerance and on every
+// kernel route in tests/test_gpu_fast_modes.py; the classes and the knife-edge rules are tests/fast_tolerance.py):
 //   RTB_F64_FAST: positions 1e-11 * L, directions 1e-12, phase 1e-12 relative (100x looser for high-NA perfect-lens
 //                 systems); NaN masks equal except knife-edge rays.
 //   RTB_F32_FAST:
@@ -25,7 +26,9 @@
 //   directions |dd| <= 2e-6
 //   phase      |dphi| <= 2e-6 * |phi|  (i.e. optical path length to 2e-6 relative)
 //   (10x looser, 2e-5, for high-NA perfect-lens systems such as the ideal OPM, where sin(theta) reaches 0.96 and the
-//   fp32 direction error is amplified by 1/cos(theta))
+//   fp32 direction error is amplified by 1/cos(theta)); phase 10x looser where fp32 t meets a small accumulated
+//   phase: long trains of large spheres (the fp32 root, <= |R|, is off by up to |R| 2^-22) and systems of long-focal-
+//   length perfect lenses (two plane steps per lens with fp32 t, |t| ~ n f): tests/fast_tolerance.py PHASE_F32
 //   validity   identical NaN masks except for rays within the position tolerance of an aperture edge, of a
 //              grazing / missing intersection or of the critical angle.
 // This translation unit is compiled with FMA contraction enabled (see Makefile).
@@ -149,7 +152,8 @@ __device__ __forceinline__ bool lens_step(const DevSurface &s, const RayT<T> &in
     to_plane_f(in, f.nx, f.ny, f.nz, fx, fy, fz, k * n1, ax, ay, az, ph_ffp);
 
     const T rnd = dot3f(in.dx, in.dy, in.dz, f.nx, f.ny, f.nz);
-    T px = fma_t(-rnd, f.nx, in.dx), py = fma_t(-rnd, f.ny, in.dy), pz = fma_t(-rnd, f.nz, in.dz);
+    const T qx = fma_t(-rnd, f.nx, in.dx), qy = fma_t(-rnd, f.ny, in.dy), qz = fma_t(-rnd, f.nz, in.dz);
+    T px = qx, py = qy, pz = qz;
     const T pn = sqrt_t(dot3f(px, py, pz, px, py, pz));
     if (pn > (T)1e-12) {
         const T inv = div_t((T)1, pn);
@@ -162,7 +166,11 @@ __device__ __forceinline__ bool lens_step(const DevSurface &s, const RayT<T> &in
         const T inv = div_t((T)1, hn);
         ux *= inv; uy *= inv; uz *= inv;
     }
-    const T sin_t1 = dot3f(px, py, pz, in.dx, in.dy, in.dz);
+    // sin(theta1) = p.d with p the unit transverse direction; p is perpendicular to n, so p.d = p.q (q = d - (d.n) n,
+    // the transverse part itself).  p.q, not p.d: the rounding of q leaves p a component ~eps / |q| along n, which
+    // p.d multiplies by d.n ~ 1 -- in fp32, 2e-5 for |q| = 2.5e-3, i.e. 1e-3 of sin(theta1) and mm-scale 1e-3 errors
+    // in the image-side position n1 f sin(theta1)
+    const T sin_t1 = dot3f(px, py, pz, qx, qy, qz);
 
     RayT<T> rb;
     const double scale = n1 * s.focal_len * (double)sin_t1;
@@ -177,7 +185,8 @@ __device__ __forceinline__ bool lens_step(const DevSurface &s, const RayT<T> &in
     rb.wl = in.wl;
     const bool culled = (abs_t(sin_t1) > f.sin_alpha) || (abs_t(sin_t2) > f.sin_alpha);
     if (culled) set_nan(rb);
-    const double plane_wave = (double)dot3f(hx, hy, hz, in.dx, in.dy, in.dz);
+    // the phase stays fp64: the plane-wave term from the fp64 focal-plane height and the widened direction
+    const double plane_wave = fma(az - fz, (double)in.dz, fma(ay - fy, (double)in.dy, (ax - fx) * (double)in.dx));
     rb.ph = (ph_ffp - (k * n1) * plane_wave) + k * ((n1 * n1) * s.focal_len + (n2 * n2) * s.focal_len);
 
     to_plane_f(rb, f.nx, f.ny, f.nz, s.cx, s.cy, s.cz, k * n2, after.ox, after.oy, after.oz, after.ph);

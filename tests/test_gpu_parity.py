@@ -844,35 +844,28 @@ def test_auto_focus_ray_modes(rt, rtm, host_api):
 @pytest.mark.parametrize("name", ["relay10_script", "doublet_nlak22", "opm", "mirrors", "edge_mix", "plano_convex_3d"])
 def test_fast_modes_tolerance(name, precision, rt, rtm):
     """
-    The two fast modes against the reference history, at the tolerances stated in csrc/trace_fast.cu:
+    The two fast modes against the reference history, at the tolerances stated in csrc/trace_fast.cu (the contract is
+    tests/fast_tolerance.py):
       f32       positions 2e-6 * L (L = 1000 mm), directions 2e-6, phase 2e-6 relative
       f64_fast  positions 1e-11 * L, directions 1e-12, phase 1e-12 relative
     (10x / 100x looser for the high-NA perfect-lens system and the deliberately extreme edge-mix rays, where the
-    direction error is amplified by 1/cos(theta)); NaN masks equal except for rays that sit within tolerance of an
-    aperture edge / grazing intersection / critical angle, or that the reference culls on round-off alone.
+    direction error is amplified by 1/cos(theta)).  Every ray is within tolerance up to its first departure, and every
+    departure is explained by a knife edge of the reference at that surface: an aperture edge, a grazing or missing
+    intersection, a root or a flat at t ~ 0, the front-side cull, the critical angle, a perfect lens's NA, or the
+    reference's absolute 1e-12 on-surface test.  tests/test_gpu_fast_modes.py covers the other kernel routes.
     """
+    import fast_tolerance
     g = load_golden(name)
     system, m_in, m_out = systems.rebuild_system(g["system"], rt, rtm)
+    mats = [m_in] + list(system.materials) + [m_out]
     want = g["history"]
     got = system.ray_trace(g["rays_in"], m_in, m_out, precision=precision)
     assert got.shape == want.shape
-    flips = np.isnan(got) != np.isnan(want)
-    ray_flips = flips.any(axis=(0, 2)).mean()
-    assert ray_flips <= (0.12 if name == "edge_mix" else 0.01), f"{name}: {ray_flips:.3%} of rays changed validity"
-    ok = np.isfinite(got) & np.isfinite(want)          # rays parallel to a plane legitimately carry +-inf
-    with np.errstate(invalid="ignore"):
-        err = np.abs(got - want)
-    scale = np.abs(want)
-    hard = name in ("opm", "edge_mix")
-    if precision == "f32":
-        tol_p, tol_d, tol_ph = (2e-5 if hard else 2e-6) * 1000.0, 2e-5 if hard else 2e-6, 2e-5 if hard else 2e-6
-    else:
-        tol_p, tol_d, tol_ph = (1e-9 if hard else 1e-11) * 1000.0, 1e-10 if hard else 1e-12, 1e-10 if hard else 1e-12
-    assert err[..., 0:3][ok[..., 0:3]].max() <= tol_p
-    assert err[..., 3:6][ok[..., 3:6]].max() <= tol_d
-    ph_ok = ok[..., 6]
-    assert (err[..., 6][ph_ok] <= tol_ph * np.maximum(scale[..., 6][ph_ok], 1.0)).all()
-    assert np.array_equal(got[..., 7][ok[..., 7]], want[..., 7][ok[..., 7]])
+    rep = fast_tolerance.compare(got, want, range(want.shape[0]), precision, fast_tolerance.is_hard(name),
+                                 system.surfaces, mats)
+    print(rep.summary(name))
+    if not fast_tolerance.is_hard(name):
+        fast_tolerance.assert_minority(rep, 0.01, name)
     # the final-slab-only instantiations of the fast kernels (no per-surface slab bookkeeping, dead rays leave the loop)
     # perform the same arithmetic: same bits as the last slab of the full history
     last = system.ray_trace(g["rays_in"], m_in, m_out, precision=precision, keep="last")
